@@ -32,6 +32,11 @@ roofline   achieved = algorithmic bytes per launch (SURVEY.md 8(d)) / mean launc
 cpu_baseline  the reference path on the host cores beside the GPU number (N=1): oracle/np_port.py, the per-world
            NumPy port at the reference's granularity (kind "port"), or the unmodified reference itself when a
            reference install is present under baseline/_ref (kind "reference")
+
+--dump-outputs DIR writes what the last timed step computed, as its caller receives it, to DIR/*.npy.  Inputs are
+seeded, so two builds run with the same arguments can be compared output for output.  Run from a tree that
+__graft_entry__.build() has built, the benchmark writes nothing into it (it may be read-only); DIR is the only
+place it writes to.
 """
 import argparse
 import json
@@ -53,6 +58,7 @@ L2_BYTES = 126 * 1024 * 1024
 METRIC = "env_steps_per_sec"
 UNIT = "env-steps/s"
 REF_CHUNK = 100     # reference arm: one bench "step" = REF_CHUNK env.step calls in each process's world
+DUMP_MAX_BYTES = 64 * 1024 * 1024   # --dump-outputs: larger outputs are written as a seeded sample of worlds
 
 
 # ------------------------------------------------------------------------------------------------
@@ -97,6 +103,15 @@ def input_bytes_from_shapes(sh):
 def ring_size(input_bytes_per_env, n_env, requested=0, cap=MAX_RING, l2_multiple=L2_MULTIPLE):
     need = int(l2_multiple * L2_BYTES / (input_bytes_per_env * n_env)) + 1
     return max(3, min(need, cap), requested or 0)
+
+
+def dump_sample(n_env, bytes_per_world, max_bytes=DUMP_MAX_BYTES):
+    """worlds --dump-outputs writes: None (all of them) when they fit max_bytes, else the same seeded sorted sample on
+    every run, so that two builds can be compared array for array"""
+    if n_env * bytes_per_world <= max_bytes:
+        return None
+    import numpy as np
+    return np.sort(np.random.RandomState(0).choice(n_env, max_bytes // bytes_per_world, replace=False))
 
 
 def workload_config(scenario, kw, n_env, n_agents, bytes_per_env, input_bytes_per_env, n_gpus, ring):
@@ -526,6 +541,7 @@ class Ring(object):
             if graph.ev:
                 graph.ev[1].record(self.stream)
         self.launches = before      # capture is not execution
+        graph.last_slot = (first + count - 1) % self.R
         self._graphs[key] = graph
         return graph
 
@@ -549,6 +565,20 @@ class Ring(object):
         if rem:
             rem_graph.replay()
             self.launches += rem
+
+    def last_outputs(self, plan):
+        """host float32 copies of what the last step of `plan` handed its caller: obs_<i> [n, obs_dim_i], rew_<i> [n],
+        done_<i> [n] per agent, restricted to dump_sample's worlds"""
+        unit_graph, units, rem_graph, rem = plan
+        env, nw, acts, ptrs, flags = self.slots[(rem_graph if rem else unit_graph).last_slot]
+        A = nw.n_agents
+        arrays = {"obs_%d" % i: o for i, o in enumerate(nw.out.obs)}
+        arrays.update(("rew_%d" % i, nw.out.rew[i]) for i in range(A))
+        arrays.update(("done_%d" % i, nw.out.done[i]) for i in range(A))
+        rows = dump_sample(self.n_env, 4 * (sum(nw.obs_dims) + 2 * A))
+        if rows is not None:
+            rows = self.torch.as_tensor(rows, device=self.dev)
+        return {k: (t if rows is None else t.index_select(0, rows)).float().cpu().numpy() for k, t in arrays.items()}
 
     def timed(self, plan, spin_cycles):
         """seconds of device time for one run of `plan`, measured between two events on the launching stream; a spin
@@ -732,6 +762,8 @@ def run_b200_arm(args, rank, local_rank, world):
     clocks = sampler.stop(t0, t1)
     total_steps, max_seconds, per_rank = aggregate_counters(N_ENV * K, seconds)
     value = total_steps / max_seconds
+    # copied now: the extras below step the same ring slots again
+    dumped = ring.last_outputs(plan) if args.dump_outputs and rank == 0 else None
 
     # ---- extras on the same K steps: two batches in flight; isolated launch; size-matched streaming kernel ----
     plan2 = ring.plan(K, two_streams=True, lead=W)
@@ -855,6 +887,11 @@ def run_b200_arm(args, rank, local_rank, world):
         }
         if cpu is not None:
             line["cpu_baseline"] = cpu
+        if dumped is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -872,12 +909,20 @@ def parse_args(argv=None):
     ap.add_argument("--scenario", default="simple_spread", help="other BASELINE configs: simple_tag, simple_world_comm, ...")
     ap.add_argument("--num-envs", type=int, default=65536, help="worlds per GPU")
     ap.add_argument("--num-agents", type=int, default=None, help="simple_spread only (N agents = N landmarks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (obs_<i> / rew_<i> / done_<i> "
+                         "per agent, float32) as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     args.scenario_kw = {"num_agents": args.num_agents} if args.num_agents is not None else {}
     return args
 
 
 def main():
+    sys.dont_write_bytecode = True      # no __pycache__ in the source tree, which may be read-only
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -20,7 +20,11 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", "..", "oracle"))
+sys.path.insert(0, os.path.join(HERE, ".."))
 import refshim  # noqa: E402
+from helpers import PER_WORLD  # noqa: E402
+
+MAX_FILE_BYTES = 1000000   # a fixture that would be larger is stored as <tag>.part<k>.npz, split along the worlds
 
 # (scenario, entity-count override, worlds W, recorded steps T): W x T >= 1536 reference steps per scenario
 CONFIGS = [
@@ -203,6 +207,20 @@ def kat():
     return out
 
 
+def save(tag, data):
+    path = os.path.join(HERE, tag + ".npz")
+    np.savez_compressed(path, **data)
+    parts = -(-os.path.getsize(path) // (MAX_FILE_BYTES * 9 // 10))      # 10 % headroom: parts differ in size
+    if parts == 1:
+        return
+    os.remove(path)
+    bounds = np.linspace(0, len(data["pv0"]), parts + 1).astype(int)
+    for k in range(parts):
+        part_path = os.path.join(HERE, "%s.part%d.npz" % (tag, k))
+        np.savez_compressed(part_path, **{key: v[bounds[k]:bounds[k + 1]] if key in PER_WORLD else v for key, v in data.items()})
+        assert os.path.getsize(part_path) < MAX_FILE_BYTES, part_path
+
+
 def main():
     only = sys.argv[1:]
     for idx, (name, n, W, T) in enumerate(CONFIGS):
@@ -210,17 +228,17 @@ def main():
             continue
         tag = name + ("_n%d" % n if n else "")
         data = run_config(name, n, W, T, seed=SEEDS[tag])
-        np.savez_compressed(os.path.join(HERE, tag + ".npz"), **data)
+        save(tag, data)
         print(tag, {k: v.shape for k, v in data.items() if not k.startswith("prop_")})
     if only:
         return
     data = run_config("simple_tag", None, 64, 8, seed=77, force_discrete=True)
-    np.savez_compressed(os.path.join(HERE, "simple_tag_force_discrete.npz"), **data)
+    save("simple_tag_force_discrete", data)
     data = run_config("simple_tag", None, 64, 8, seed=78, discrete_input=True)
-    np.savez_compressed(os.path.join(HERE, "simple_tag_discrete_input.npz"), **data)
+    save("simple_tag_discrete_input", data)
     for counts, tag in (((1, 1, 2), "simple_tag_1v1"), ((4, 2, 2), "simple_tag_4v2"), ((6, 2, 3), "simple_tag_6v2")):
         data = run_config("simple_tag", counts, 64, 6, seed=80 + counts[0])     # entity-count variants
-        np.savez_compressed(os.path.join(HERE, tag + ".npz"), **data)
+        save(tag, data)
     np.savez_compressed(os.path.join(HERE, "kat.npz"), **kat())
 
 

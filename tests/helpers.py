@@ -1,4 +1,5 @@
 """shared test helpers (the oracle is imported HERE, in tests/, only as the checker)"""
+import glob
 import os
 
 import numpy as np
@@ -29,8 +30,22 @@ VARIANTS = {
 NO_BENCHMARK = ("simple", "simple_push", "simple_speaker_listener", "simple_reference")
 
 
+# arrays of a fixture with one row per recorded world; the rest (prop_*, flags) describe the whole scenario
+PER_WORLD = ("pv0", "lm", "comm0", "goal", "act", "pv", "comm", "obs", "rew", "done", "info")
+
+
 def load_golden(tag):
-    return dict(np.load(os.path.join(GOLDEN, tag + ".npz")))
+    """one fixture; a fixture stored as <tag>.part<k>.npz (each file stays below 1 MB) is joined along the worlds"""
+    path = os.path.join(GOLDEN, tag + ".npz")
+    if os.path.exists(path):
+        return dict(np.load(path))
+    parts = [dict(np.load(p)) for p in sorted(glob.glob(os.path.join(GOLDEN, tag + ".part*.npz")))]
+    if not parts:
+        raise FileNotFoundError(path)
+    g = parts[0]
+    for k in PER_WORLD:
+        g[k] = np.concatenate([p[k] for p in parts])
+    return g
 
 
 def make_product_env(tag, **kw):

@@ -303,3 +303,18 @@ def test_bench_numa_pinning_degrades_gracefully():
         assert os.sched_getaffinity(0) <= before
     finally:
         os.sched_setaffinity(0, before)
+
+
+def test_bench_dump_outputs_arguments_and_sample():
+    """--dump-outputs takes a directory; outputs over 64 MB are written as one fixed sample of worlds; a run must time
+    at least one step"""
+    sys.path.insert(0, ROOT)
+    import bench
+    assert bench.parse_args(["--steps", "7", "--dump-outputs", "out"]).dump_outputs == "out"
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        with pytest.raises(SystemExit):
+            bench.parse_args(bad)
+    assert bench.dump_sample(65536, 4 * (3 * 18 + 2 * 3)) is None          # the headline workload: every world
+    rows = bench.dump_sample(1 << 20, 1024)
+    assert rows.size == bench.DUMP_MAX_BYTES // 1024 and rows[-1] < 1 << 20 and (np.diff(rows) > 0).all()
+    assert np.array_equal(rows, bench.dump_sample(1 << 20, 1024))

@@ -305,3 +305,31 @@ def test_closed_loop_policy_rollout(tag, n, T, H):
     with pytest.raises(MpeError):
         env_w.rollout_policy([(torch.zeros(32, od, device="cuda"), torch.zeros(32, device="cuda"), torch.zeros(5, 32, device="cuda"),
                                torch.zeros(5, device="cuda")) for od in env_w.world.native.obs_dims], 2)
+
+
+def test_bench_dump_outputs_repeat_exactly(tmp_path):
+    """bench.py --dump-outputs writes what the last timed step returned (per agent: obs, rew, done as float32), and two
+    runs with the same arguments write the same arrays"""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n = 4096
+    dumps = []
+    for r in range(2):
+        d = tmp_path / str(r)
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "30", "--warmup", "3",
+                              "--num-envs", str(n), "--cpu-seconds", "0", "--e2e-steps", "3", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=900, cwd=root)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 30
+        dumps.append({p.name[:-4]: np.load(p) for p in d.iterdir()})
+    a, b = dumps
+    assert sorted(a) == sorted("%s_%d" % (k, i) for k in ("obs", "rew", "done") for i in range(3))
+    for k in a:
+        assert a[k].dtype == np.float32 and a[k].shape[0] == n and np.array_equal(a[k], b[k]), k
+        assert np.isfinite(a[k]).all(), k
+    assert a["obs_0"].shape == (n, 18)
+    assert np.array_equal(a["rew_0"], a["rew_1"]) and np.array_equal(a["rew_0"], a["rew_2"])     # shared reward
+    assert set(np.unique(a["done_0"])) <= {0.0, 1.0}
