@@ -80,10 +80,11 @@ enum mpe_step_flags {
                                            [n_env][n_sub_i], one index per sub-action -- movement (0 none, 1 -x,
                                            2 +x, 3 -y, 4 +y) if the agent is movable, then the utterance
                                            (one-hot of the index) if it is not silent; decoded inside the kernel */
-    MPE_FLAG_HOST_SLAB = 8              /* mpe_step_host only: obs_n_host[0..A), rew_host, done_host (, info_host)
+    MPE_FLAG_HOST_SLAB = 8,             /* mpe_step_host only: obs_n_host[0..A), rew_host, done_host (, info_host)
                                            are consecutive parts of ONE host allocation and their device
                                            counterparts of ONE device allocation, with equal gaps < 512 B:
                                            the D2H copies are coalesced into a single DMA */
+    MPE_FLAG_SAMPLE_ACTIONS = 16        /* mpe_collect only: act with MADDPG's Gumbel-softmax exploration sample */
 };
 
 /*
@@ -205,6 +206,40 @@ MPE_API int mpe_rollout_policy(mpe_handle h, void *agent_pv_dev, const void *lm_
                                const float *const *w2_n, const float *const *b2_n, int32_t hidden, int32_t n_steps,
                                float *const *obs_n_dev, float *rew_sum_dev, float *rew_steps_dev,
                                float *const *act_record_n, uint8_t *done_dev, uint32_t flags, void *stream);
+
+/* Training experience in ONE launch: the closed loop of mpe_rollout_policy, with a one- or two-hidden-layer actor,
+ * optional exploration noise and a record of every step's observations -- everything a replay buffer needs:
+ * (obs_record[t], act_record[t], rew_steps[t], obs_record[t + 1]), with obs_n_dev holding the observation after the
+ * last step.
+ *   depth 1:  a_i = softmax(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i)                          (obs_dim_i -> H -> 5)
+ *   depth 2:  a_i = softmax(W3_i . relu(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i) + b3_i)      (obs_dim_i -> H -> H -> 5,
+ *             the MADDPG actor: fc 64 relu, fc 64 relu, fc 5)
+ * hidden = H = 32 or 64.  Weights, all 16-byte aligned except b2 / b3 (4-byte):
+ *   w1_n[i] float [obs_dim_i][H] (input-major, W1^T of a torch Linear(obs_dim_i, H)), b1_n[i] [H];
+ *   depth 1: w2_n[i] [5][H], b2_n[i] [5], w3_n = b3_n = NULL;
+ *   depth 2: w2_n[i] [H][H] (torch Linear(H, H).weight), b2_n[i] [H], w3_n[i] [5][H], b3_n[i] [5].
+ * Every unit sums bias + inputs in ascending input order with FMAs.
+ * flags: MPE_FLAG_SHARED_REWARD as for mpe_step; MPE_FLAG_SAMPLE_ACTIONS replaces softmax(logits) by the exploration
+ * sample softmax(logits - log(-log u)), u = (2 (bits >> 9) + 1) 2^-24 from Philox4x32-10 with key (sample_seed lo, hi)
+ * and counter (w lo, w hi, sample_step + t, 0x40000000 | agent << 1 | block), w = world_offset + world index, blocks 0
+ * and 1 giving words 0-3 and 4 for the five logits.  Draws depend on the global world index and the global step only,
+ * so a sharded batch or a rollout split into several calls draws exactly what one call over the whole batch draws.
+ * Records (NULL, or per agent): act_record_n[i] float [n_steps][n_env][5], the actions taken (sampled ones when
+ * sampling); obs_record_n[i] float [n_steps][n_env][obs_dim_i] (16-byte aligned, all agents or none), row t = the
+ * observation agent i acted on at step t (row 0 = the state before the call).  Feeding act_record_n to mpe_step
+ * reproduces state, observations and rewards bit for bit.  Outputs otherwise as mpe_rollout_policy.
+ * Errors: MPE_ERR_BAD_ARG for NULL / misaligned pointers, depth not 1 or 2, hidden not 32 or 64, n_steps < 0 or
+ * sample_step + n_steps > 2^32; MPE_ERR_NO_DEVICE for a device-less handle; MPE_ERR_UNSUPPORTED for a scenario
+ * without the kernel (as mpe_rollout_policy) or MPE_FLAG_FORCE_DISCRETE_ACTION / MPE_FLAG_DISCRETE_ACTION_INPUT. */
+MPE_API int mpe_collect(mpe_handle h, void *agent_pv_dev, const void *lm_p_dev, float *comm_dev, const int32_t *goal_dev,
+                        int32_t depth, int32_t hidden,
+                        const float *const *w1_n, const float *const *b1_n,
+                        const float *const *w2_n, const float *const *b2_n,
+                        const float *const *w3_n, const float *const *b3_n,
+                        int32_t n_steps, uint64_t sample_seed, uint32_t sample_step, uint64_t world_offset,
+                        float *const *obs_n_dev, float *rew_sum_dev, float *rew_steps_dev,
+                        float *const *act_record_n, float *const *obs_record_n, uint8_t *done_dev,
+                        uint32_t flags, void *stream);
 
 /* Same step for a caller that holds HOST buffers (what the reference's callers hold):
  * act_n_host[i] -> (async H2D into act_n_dev[i]) -> mpe_step -> (async D2H) obs_n_host[i],

@@ -23,8 +23,11 @@ FLAG_SHARED_REWARD = 1
 FLAG_FORCE_DISCRETE_ACTION = 2
 FLAG_DISCRETE_ACTION_INPUT = 4
 FLAG_HOST_SLAB = 8
+FLAG_SAMPLE_ACTIONS = 16
 
+ERR_BAD_ARG = -1
 ERR_UNSUPPORTED = -3
+ERR_NO_DEVICE = -5
 
 
 class MpeDesc(ctypes.Structure):
@@ -86,6 +89,9 @@ _SIGNATURES = {
     "mpe_rollout": (ctypes.c_int, [_P, _P, _P, _P, _P, _PP, ctypes.c_int32, _PP, _P, _P, _P, ctypes.c_uint32, _P]),
     "mpe_rollout_policy": (ctypes.c_int, [_P, _P, _P, _P, _P, _PP, _PP, _PP, _PP, ctypes.c_int32, ctypes.c_int32, _PP, _P, _P,
                                           _PP, _P, ctypes.c_uint32, _P]),
+    "mpe_collect": (ctypes.c_int, [_P, _P, _P, _P, _P, ctypes.c_int32, ctypes.c_int32, _PP, _PP, _PP, _PP, _PP, _PP,
+                                   ctypes.c_int32, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint64, _PP, _P, _P, _PP, _PP,
+                                   _P, ctypes.c_uint32, _P]),
     "mpe_step_host": (ctypes.c_int, [_P, _P, _P, _P, _P, _PP, _PP, _PP, _P, _P, _P, _PP, _P, _P, _P,
                                      ctypes.c_uint32, _P]),
     "mpe_strerror": (ctypes.c_char_p, [ctypes.c_int]),

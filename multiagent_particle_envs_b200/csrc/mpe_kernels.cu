@@ -250,8 +250,9 @@ __device__ __forceinline__ void decode_rows(const float *s_act, int lane, const 
     });
 }
 
-// observation rows of one 32-world tile: full warps write through the warp-private tiles and stream them out as
-// coalesced 16-byte stores; the batch's last, partial warp writes its rows straight to global memory.
+// observation rows of one 32-world tile into obs[i] + (row0 + world) * obs_dim_i: with `tile` (a full warp whose rows
+// start 16-byte aligned) the rows go through the warp-private tiles and stream out as coalesced 16-byte stores;
+// otherwise (the batch's last, partial warp) each lane writes its row straight to global memory.
 // `half` < 0: every agent; 0: agents [0, split_point); 1: agents [split_point, A) (warp pairs; the second warp also
 // computes the rewards, so it gets the smaller share: split_point = ceil(2A/3)).
 template <class P>
@@ -259,10 +260,11 @@ __host__ __device__ constexpr int split_point() { return (2 * P::A + 2) / 3; }
 template <class P>
 __host__ __device__ constexpr int agent_half(int i) { return i < split_point<P>() ? 0 : 1; }
 template <class P>
-__device__ __forceinline__ void write_observations(const StepArgs &a, const DevDesc &d, const typename P::W &w, float *s_warp,
-                                                   int lane, int rows, bool active, int64_t w0, int64_t wi, int half) {
+__device__ __forceinline__ void write_observations(float *const *obs, int64_t row0, const DevDesc &d, const typename P::W &w,
+                                                   float *s_warp, int lane, bool tile, bool active, int64_t w0, int64_t wi,
+                                                   int half) {
     constexpr int A = P::A;
-    if (rows == 32) {
+    if (tile) {
         // Tiles are private per agent (dense ones), so no barrier is needed between agents: all rows are
         // written, one __syncwarp, then the warp streams every tile out as 16-byte stores and retires.
         // (A TMA bulk store was measured slower here: the warp has to stay resident until the copy
@@ -275,7 +277,7 @@ __device__ __forceinline__ void write_observations(const StepArgs &a, const DevD
             P::template observe<i>(d, w, o);
             if constexpr (!Shape<P>::obs_private(i)) {  // tiles without a slot of their own share one
                 __syncwarp();
-                obs_tile_store<OD>(a.obs[i] + w0 * OD, s_warp + Shape<P>::obs_off(i), lane);
+                obs_tile_store<OD>(obs[i] + (row0 + w0) * OD, s_warp + Shape<P>::obs_off(i), lane);
                 __syncwarp();
             }
         });
@@ -284,13 +286,13 @@ __device__ __forceinline__ void write_observations(const StepArgs &a, const DevD
             constexpr int i = decltype(ic)::value;
             constexpr int OD = P::obs_dim(i);
             if (half >= 0 && agent_half<P>(i) != half) return;
-            if constexpr (Shape<P>::obs_private(i)) obs_tile_store<OD>(a.obs[i] + w0 * OD, s_warp + Shape<P>::obs_off(i), lane);
+            if constexpr (Shape<P>::obs_private(i)) obs_tile_store<OD>(obs[i] + (row0 + w0) * OD, s_warp + Shape<P>::obs_off(i), lane);
         });
-    } else if (active) {  // the batch's last, partial warp: rows go straight to global memory
+    } else if (active) {
         static_for<A>([&](auto ic) {
             constexpr int i = decltype(ic)::value;
             if (half >= 0 && agent_half<P>(i) != half) return;
-            RowWriter o{a.obs[i] + wi * P::obs_dim(i)};
+            RowWriter o{obs[i] + (row0 + wi) * P::obs_dim(i)};
             P::template observe<i>(d, w, o);
         });
     }
@@ -533,7 +535,7 @@ __global__ void __launch_bounds__(DENSE ? 128 : MPE_BOUND_THREADS, DENSE ? 6 : M
     }
     if constexpr (SPLIT) pair_sync(1 + (warp >> 1));   // the partner has consumed the exchange buffer (= obs tiles of the even warp)
     if (!(a.flags & (kFlagPdlEarly | kFlagPdlAfterLoads | kFlagPdlAtExit | kFlagPdlAfterIssue))) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    write_observations<P>(a, d, w, s_warp, lane, rows, active, w0, wi, SPLIT ? half : -1);
+    write_observations<P>(a.obs, 0, d, w, s_warp, lane, rows == 32, active, w0, wi, SPLIT ? half : -1);
     if (active && (!SPLIT || half == 1)) {
 #pragma unroll
         for (int i = 0; i < A; ++i) {
@@ -649,7 +651,7 @@ __global__ void __launch_bounds__(MPE_BOUND_THREADS, MPE_MIN_BLOCKS) mpe_pipe_ke
 #pragma unroll
             for (int i = 0; i < A; ++i) rew[i] = sum;
         }
-        write_observations<P>(a, d, w, s_warp, lane, 32, true, w0, wi, -1);
+        write_observations<P>(a.obs, 0, d, w, s_warp, lane, true, true, w0, wi, -1);
 #pragma unroll
         for (int i = 0; i < A; ++i) {
             a.rew[i * n + wi] = rew[i];
@@ -777,7 +779,7 @@ __global__ void __launch_bounds__(MPE_BOUND_THREADS, MPE_MIN_BLOCKS) mpe_rollout
         for (int q = 0; q < NC; ++q) a.comm[q * n + wi] = w.c[q];
     }
     P::prepare(d, w);
-    write_observations<P>(a, d, w, s_warp, lane, rows, active, w0, wi, -1);
+    write_observations<P>(a.obs, 0, d, w, s_warp, lane, rows == 32, active, w0, wi, -1);
     if (active) {
 #pragma unroll
         for (int i = 0; i < A; ++i) {
@@ -791,11 +793,14 @@ __global__ void __launch_bounds__(MPE_BOUND_THREADS, MPE_MIN_BLOCKS) mpe_rollout
 // ---- K-step CLOSED-LOOP rollout with an in-kernel policy (SURVEY.md 8(f) rank 3, the persistent form with a device-
 // resident policy; VERDICT r1 item 9) -------------------------------------------------------------------------------
 // T consecutive MultiAgentEnv.step calls in ONE launch where every agent's action is produced inside the kernel by its
-// own two-layer perceptron  a_i = softmax(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i)  (obs_dim_i -> H -> 5 movement
-// probabilities, the MADDPG actor shape).  A world's state lives in registers for all T steps; an agent's observation
-// is produced straight into registers (never written), pushed through the perceptron (weights of all agents sit in
-// shared memory once per block, read as broadcast LDS.128), decoded and integrated.  Per step NOTHING is read from HBM
-// and only the optional records (rewards, actions) are written; observations are written for the final state.
+// own perceptron.  DEPTH 1:  a_i = softmax(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i)  (obs_dim_i -> H -> 5 movement
+// probabilities); DEPTH 2, the MADDPG actor:  a_i = softmax(W3_i . relu(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i) + b3_i)
+// (obs_dim_i -> H -> H -> 5).  A world's state lives in registers for all T steps; an agent's observation is produced
+// straight into registers, pushed through the perceptron (weights of all agents sit in shared memory once per block,
+// read as broadcast LDS.128), decoded and integrated.  Per step NOTHING is read from HBM and only the optional records
+// (rewards, actions, observations) are written; observations are always written for the final state.
+// With MPE_FLAG_SAMPLE_ACTIONS the action is MADDPG's exploration sample softmax(logits + g), g = -log(-log u) Gumbel
+// noise from a Philox stream keyed by (seed, global world, step, agent), so trajectories do not depend on sharding.
 // Scenarios whose agents all move and are silent (simple_spread, simple_tag, ...).  The physics / reward / observation
 // arithmetic is the fused step's: feeding the recorded actions to T fused steps reproduces the final state, the
 // observations and the reward sums bit for bit; the perceptron matches a float64 evaluation to ~1e-6 (tests).
@@ -804,15 +809,26 @@ struct PolicyArgs {
     int32_t T;
     float *rew_steps;               // [T][A][n] or null
     float *act_rec[kMaxA];          // [T][n][5] per agent, or null
+    float *obs_rec[kMaxA];          // [T][n][obs_dim_i] per agent (row t: the observation acted on at step t), or all null
     const float *w1[kMaxA];         // [obs_dim_i][H]  (input-major: W1^T of a torch Linear(obs_dim_i, H))
     const float *b1[kMaxA];         // [H]
-    const float *w2[kMaxA];         // [5][H]          (the layout of a torch Linear(H, 5).weight)
-    const float *b2[kMaxA];         // [5]
+    const float *w2[kMaxA];         // depth 1: [5][H] (torch Linear(H, 5).weight); depth 2: [H][H] (Linear(H, H).weight)
+    const float *b2[kMaxA];         // depth 1: [5]; depth 2: [H]
+    const float *w3[kMaxA];         // depth 2: [5][H] (torch Linear(H, 5).weight); depth 1: unused
+    const float *b3[kMaxA];         // depth 2: [5]
+    uint2 sample_key;               // Philox key of the exploration noise (MPE_FLAG_SAMPLE_ACTIONS)
+    uint64_t world_offset;          // global index of world 0 of this batch
+    uint32_t sample_step;           // global step index of step 0 of this launch
 };
 
-template <class P, int H>
+// shared-memory image of one agent's actor (floats, every part 16-byte aligned):
+//   depth 1: [W1: OD x H][b1: H][W2: 5 x H][b2: 5, padded to 8]
+//   depth 2: [W1: OD x H][b1: H][W2: H x H][b2: H][W3: H x 8, input-major, outputs 5..7 zero][b3: 5, padded to 8]
+template <class P, int H, int DEPTH>
 struct PolicyShape {
-    __host__ __device__ static constexpr int agent_floats(int i) { return P::obs_dim(i) * H + H + 5 * H + 8; }
+    __host__ __device__ static constexpr int agent_floats(int i) {
+        return P::obs_dim(i) * H + H + (DEPTH == 1 ? 5 * H + 8 : H * H + H + 8 * H + 8);
+    }
     __host__ __device__ static constexpr int agent_off(int i) { int s = 0; for (int j = 0; j < i; ++j) s += agent_floats(j); return s; }
     static constexpr int kWeightFloats = (agent_off(P::A) + 3) & ~3;
 };
@@ -827,15 +843,21 @@ struct RegWriter {
     __device__ __forceinline__ void put2(float2 a) { put2(a.x, a.y); }
 };
 
+// Philox counter word 3 of the exploration noise: bit 30 set keeps it apart from the reset stream (small block numbers
+// and 0x80000000); two blocks per (world, step, agent), 5 of their 8 words used
+__host__ __device__ constexpr uint32_t sample_tag(int agent, int block) { return 0x40000000u | (static_cast<uint32_t>(agent) << 1) | block; }
 
-// one agent of the in-kernel policy: observation -> registers -> two-layer perceptron -> softmax -> decoded (u.x, u.y).
-// A plain force-inlined function with unrolled loops (not a lambda: arrays captured by reference by a lambda that the
-// compiler declines to inline end up in local memory).  W = [W1: OD x H][b1: H][W2: 5 x H][b2: 5] in shared memory.
-template <class P, int H, int I>
+// one agent of the in-kernel policy: observation -> registers -> perceptron -> (+ Gumbel noise) -> softmax -> decoded
+// (u.x, u.y).  A plain force-inlined function with unrolled loops (not a lambda: arrays captured by reference by a lambda
+// that the compiler declines to inline end up in local memory).  W = the agent's PolicyShape image in shared memory.
+// Summation order (fixed; the float64 tests rely on it): every unit starts from its bias and adds its inputs in
+// ascending order with FMAs -- layer 1 over j = observation index, layer 2 over j = layer-1 unit, the output layer over
+// q = last hidden unit.
+template <class P, int H, int DEPTH, int I>
 __device__ __forceinline__ float2 policy_agent(const DevDesc &d, const typename P::W &w, const float *__restrict__ W,
-                                               float *__restrict__ record) {
+                                               float *__restrict__ record, bool sample, uint2 key, uint64_t gw, uint32_t step) {
     constexpr int OD = P::obs_dim(I);
-    const float *W1 = W, *B1 = W1 + OD * H, *W2 = B1 + H, *B2 = W2 + 5 * H;
+    const float *W1 = W, *B1 = W1 + OD * H, *W2 = B1 + H;
     RegWriter<OD> o;
     P::template observe<I>(d, w, o);                       // scenario.observation(agent I) -> registers
     float h[H];
@@ -859,18 +881,63 @@ __device__ __forceinline__ float2 policy_agent(const DevDesc &d, const typename 
 #pragma unroll
     for (int q = 0; q < H; ++q) h[q] = fmaxf(h[q], 0.0f);  // ReLU
     float lg[5];
+    if constexpr (DEPTH == 1) {
+        const float *B2 = W2 + 5 * H;
 #pragma unroll
-    for (int c = 0; c < 5; ++c) {                          // logits[c] = b2[c] + sum_q h[q] * W2[c][q]  (ascending q)
-        float acc = B2[c];
+        for (int c = 0; c < 5; ++c) {                      // logits[c] = b2[c] + sum_q h[q] * W2[c][q]  (ascending q)
+            float acc = B2[c];
 #pragma unroll
-        for (int q = 0; q < H; q += 4) {
-            const float4 wv = *reinterpret_cast<const float4 *>(W2 + c * H + q);
-            acc = __fmaf_rn(h[q], wv.x, acc);
-            acc = __fmaf_rn(h[q + 1], wv.y, acc);
-            acc = __fmaf_rn(h[q + 2], wv.z, acc);
-            acc = __fmaf_rn(h[q + 3], wv.w, acc);
+            for (int q = 0; q < H; q += 4) {
+                const float4 wv = *reinterpret_cast<const float4 *>(W2 + c * H + q);
+                acc = __fmaf_rn(h[q], wv.x, acc);
+                acc = __fmaf_rn(h[q + 1], wv.y, acc);
+                acc = __fmaf_rn(h[q + 2], wv.z, acc);
+                acc = __fmaf_rn(h[q + 3], wv.w, acc);
+            }
+            lg[c] = acc;
         }
-        lg[c] = acc;
+    } else {
+        // The second hidden layer is never materialised: unit q is computed, rectified and immediately folded into the
+        // five logits, so only h[H] and lg[5] stay live (the register profile of depth 1).  The q loop stays rolled
+        // (H x H unrolled FMAs per agent would overflow the instruction cache); the j loop is unrolled because h needs
+        // compile-time indices.  h2_q = relu(b2[q] + sum_j h[j] W2[q][j]) (ascending j), then
+        // logits[c] = b3[c] + sum_q h2_q W3[c][q] (ascending q).
+        const float *B2 = W2 + H * H, *W3 = B2 + H, *B3 = W3 + 8 * H;
+#pragma unroll
+        for (int c = 0; c < 5; ++c) lg[c] = B3[c];
+#pragma unroll 1
+        for (int q = 0; q < H; ++q) {
+            const float *row = W2 + q * H;
+            float acc = B2[q];
+#pragma unroll
+            for (int j = 0; j < H; j += 4) {
+                const float4 wv = *reinterpret_cast<const float4 *>(row + j);
+                acc = __fmaf_rn(h[j], wv.x, acc);
+                acc = __fmaf_rn(h[j + 1], wv.y, acc);
+                acc = __fmaf_rn(h[j + 2], wv.z, acc);
+                acc = __fmaf_rn(h[j + 3], wv.w, acc);
+            }
+            acc = fmaxf(acc, 0.0f);
+            const float4 wa = *reinterpret_cast<const float4 *>(W3 + 8 * q);
+            const float4 wb = *reinterpret_cast<const float4 *>(W3 + 8 * q + 4);
+            lg[0] = __fmaf_rn(acc, wa.x, lg[0]);
+            lg[1] = __fmaf_rn(acc, wa.y, lg[1]);
+            lg[2] = __fmaf_rn(acc, wa.z, lg[2]);
+            lg[3] = __fmaf_rn(acc, wa.w, lg[3]);
+            lg[4] = __fmaf_rn(acc, wb.x, lg[4]);
+        }
+    }
+    if (sample) {   // MADDPG's exploration: softmax(logits - log(-log u)), u uniform in (0, 1)
+        const uint4 ctr = make_uint4(static_cast<uint32_t>(gw), static_cast<uint32_t>(gw >> 32), step, sample_tag(I, 0));
+        const uint4 r0 = philox4x32_10(ctr, key);
+        const uint4 r1 = philox4x32_10(make_uint4(ctr.x, ctr.y, ctr.z, sample_tag(I, 1)), key);
+        const uint32_t bits[5] = {r0.x, r0.y, r0.z, r0.w, r1.x};
+#pragma unroll
+        for (int c = 0; c < 5; ++c) {
+            // (2 k + 1) 2^-24, k < 2^23: exact in fp32 and strictly inside (0, 1), so both logarithms are finite
+            const float u = static_cast<float>(2u * (bits[c] >> 9) + 1u) * 5.9604644775390625e-8f;
+            lg[c] = __fadd_rn(lg[c], -logf(-logf(u)));
+        }
     }
     const float m = fmaxf(fmaxf(fmaxf(lg[0], lg[1]), fmaxf(lg[2], lg[3])), lg[4]);
     float e[5], sum = 0.0f;
@@ -890,11 +957,20 @@ __device__ __forceinline__ float2 policy_agent(const DevDesc &d, const typename 
     return make_float2(__fmul_rn(x, d.a_sens[I]), __fmul_rn(y, d.a_sens[I]));
 }
 
-template <class P, int H>
-__global__ void __launch_bounds__(128) mpe_policy_rollout_kernel(const __grid_constant__ PolicyArgs pa) {
+// block sizes: depth 1 as it always was (1, 2 or 4 warps); depth 2 up to 8 warps, because its weights (70-92 KB at
+// H = 64) are staged once per block and only larger blocks let an SM hold as many warps as its registers allow
+template <int DEPTH>
+constexpr int kPolicyMaxWarps = DEPTH == 1 ? 4 : 8;
+
+// EXTRAS = false: the plain closed loop (no exploration noise, no observation records) compiled without those paths.
+// With them the depth-1 tag kernel at H = 64 needs 189 registers instead of 160 and takes 40.4 instead of 34.2 us per
+// step at 65 536 worlds (B200, 1000 W), so depth 1 keeps the plain build for plain calls.
+template <class P, int H, int DEPTH, bool EXTRAS>
+__global__ void __launch_bounds__(32 * kPolicyMaxWarps<DEPTH>) mpe_policy_rollout_kernel(const __grid_constant__ PolicyArgs pa) {
     static_assert(P::NS == 0 && H % 4 == 0, "policy rollout: silent agents, hidden width a multiple of 4");
+    static_assert(DEPTH == 1 || DEPTH == 2, "policy rollout: one or two hidden layers");
     constexpr int A = P::A, L = P::L;
-    using PS = PolicyShape<P, H>;
+    using PS = PolicyShape<P, H, DEPTH>;
     const StepArgs &a = pa.s;
     extern __shared__ __align__(16) float smem[];
     float *s_w = smem;
@@ -906,8 +982,18 @@ __global__ void __launch_bounds__(128) mpe_policy_rollout_kernel(const __grid_co
         float *base = s_w + PS::agent_off(i);
         for (int q = threadIdx.x; q < OD * H; q += blockDim.x) base[q] = pa.w1[i][q];
         for (int q = threadIdx.x; q < H; q += blockDim.x) base[OD * H + q] = pa.b1[i][q];
-        for (int q = threadIdx.x; q < 5 * H; q += blockDim.x) base[OD * H + H + q] = pa.w2[i][q];
-        for (int q = threadIdx.x; q < 5; q += blockDim.x) base[OD * H + H + 5 * H + q] = pa.b2[i][q];
+        base += OD * H + H;
+        if constexpr (DEPTH == 1) {
+            for (int q = threadIdx.x; q < 5 * H; q += blockDim.x) base[q] = pa.w2[i][q];
+            for (int q = threadIdx.x; q < 5; q += blockDim.x) base[5 * H + q] = pa.b2[i][q];
+        } else {
+            for (int q = threadIdx.x; q < H * H; q += blockDim.x) base[q] = pa.w2[i][q];
+            for (int q = threadIdx.x; q < H; q += blockDim.x) base[H * H + q] = pa.b2[i][q];
+            base += H * H + H;
+            for (int q = threadIdx.x; q < 8 * H; q += blockDim.x)        // W3 [5][H] -> [H][8]
+                base[q] = (q & 7) < 5 ? pa.w3[i][(q & 7) * H + (q >> 3)] : 0.0f;
+            for (int q = threadIdx.x; q < 8; q += blockDim.x) base[8 * H + q] = q < 5 ? pa.b3[i][q] : 0.0f;
+        }
     });
     __syncthreads();
 
@@ -920,6 +1006,9 @@ __global__ void __launch_bounds__(128) mpe_policy_rollout_kernel(const __grid_co
     const int64_t wi = w0 + (active ? lane : 0);
     float *s_warp = smem + PS::kWeightFloats + warp * Shape<P>::kWarpFloats;
     const DevDesc &d = a.d;
+    const bool sample = EXTRAS && (a.flags & MPE_FLAG_SAMPLE_ACTIONS) != 0;
+    const bool rec_obs = EXTRAS && pa.obs_rec[0] != nullptr;
+    const uint64_t gw = pa.world_offset + static_cast<uint64_t>(wi);
 
     typename P::W w;
 #pragma unroll
@@ -941,14 +1030,30 @@ __global__ void __launch_bounds__(128) mpe_policy_rollout_kernel(const __grid_co
 #pragma unroll
     for (int i = 0; i < A; ++i) rsum[i] = 0.0f;
 #pragma unroll 1
-    for (int t = 0; t < pa.T; ++t) {
-        float ux[A], uy[A];
+    for (int t = 0;; ++t) {
         P::prepare(d, w);
+        const bool last = t == pa.T;
+        if (last || rec_obs) {
+            // the observations of step t go to record row t, and after the last step to obs_n: one call site for both
+            // keeps a single inlined copy of every agent's observation code.  The tile path needs every row block
+            // 16-byte aligned, which fails for odd t when n * obs_dim_i is not a multiple of 4: such rows go direct.
+            float *const *obs = last ? a.obs : pa.obs_rec;
+            const int64_t row0 = last ? 0 : static_cast<int64_t>(t) * n;
+            bool tile = rows == 32;
+#pragma unroll
+            for (int i = 0; i < A; ++i)
+                tile = tile && ((reinterpret_cast<uintptr_t>(obs[i] + (row0 + w0) * P::obs_dim(i)) & 15u) == 0);
+            write_observations<P>(obs, row0, d, w, s_warp, lane, tile, active, w0, wi, -1);
+            if (last) break;
+            __syncwarp();   // every lane has streamed the tiles out before any lane refills them
+        }
+        float ux[A], uy[A];
         static_for<A>([&](auto ic) {
             constexpr int i = decltype(ic)::value;
-            const float2 u = policy_agent<P, H, i>(d, w, s_w + PolicyShape<P, H>::agent_off(i),
-                                                   (pa.act_rec[i] != nullptr && active)
-                                                       ? pa.act_rec[i] + (static_cast<int64_t>(t) * n + wi) * 5 : nullptr);
+            const float2 u = policy_agent<P, H, DEPTH, i>(d, w, s_w + PS::agent_off(i),
+                                                          (pa.act_rec[i] != nullptr && active)
+                                                              ? pa.act_rec[i] + (static_cast<int64_t>(t) * n + wi) * 5 : nullptr,
+                                                          sample, pa.sample_key, gw, pa.sample_step + static_cast<uint32_t>(t));
             ux[i] = u.x;
             uy[i] = u.y;
         });
@@ -974,8 +1079,6 @@ __global__ void __launch_bounds__(128) mpe_policy_rollout_kernel(const __grid_co
         for (int i = 0; i < A; ++i)
             if (P::movable(i)) a.pv[i * n + wi] = make_float4(w.px[i], w.py[i], w.vx[i], w.vy[i]);
     }
-    P::prepare(d, w);
-    write_observations<P>(a, d, w, s_warp, lane, rows, active, w0, wi, -1);
     if (active) {
 #pragma unroll
         for (int i = 0; i < A; ++i) {
@@ -1199,8 +1302,9 @@ struct Program {
     KernelFn split_fn;  // fused step with a warp PAIR per 32-world tile (small batches of heavy scenarios)
     KernelFn pipe_fn;   // software-pipelined persistent fused step (null unless every action tile is dense)
     int pipe_smem;      // dynamic shared memory per WARP of the pipelined kernel
-    void (*policy_fn[2])(PolicyArgs);  // K-step closed-loop rollout, hidden width 32 / 64 (null: not built for this program)
-    int policy_weight_floats[2];
+    void (*policy_fn[2][2])(PolicyArgs);  // K-step closed-loop rollout [depth - 1][hidden 32 / 64] (null: not built)
+    void (*policy_plain_fn[2])(PolicyArgs);  // the same at depth 1 without exploration noise and observation records
+    int policy_weight_floats[2][2];
     void (*rollout_fn)(RolloutArgs);   // K-step open-loop rollout
     int rollout_smem;   // dynamic shared memory per WARP of the rollout kernel
     KernelFn lanes_fn;  // lane-per-agent fused step (simple_spread only), else null
@@ -1233,10 +1337,16 @@ static Program make_program() {
     p.rollout_smem = Shape<P>::kRolloutWarpBytes;
     // the closed-loop rollout is built for the BASELINE.json scenarios whose agents all move and are silent
     if constexpr (policy_rollout_ok<P>() && PolicyBuilt<P>::value) {
-        p.policy_fn[0] = mpe_policy_rollout_kernel<P, 32>;
-        p.policy_fn[1] = mpe_policy_rollout_kernel<P, 64>;
-        p.policy_weight_floats[0] = PolicyShape<P, 32>::kWeightFloats;
-        p.policy_weight_floats[1] = PolicyShape<P, 64>::kWeightFloats;
+        p.policy_plain_fn[0] = mpe_policy_rollout_kernel<P, 32, 1, false>;
+        p.policy_plain_fn[1] = mpe_policy_rollout_kernel<P, 64, 1, false>;
+        p.policy_fn[0][0] = mpe_policy_rollout_kernel<P, 32, 1, true>;
+        p.policy_fn[0][1] = mpe_policy_rollout_kernel<P, 64, 1, true>;
+        p.policy_fn[1][0] = mpe_policy_rollout_kernel<P, 32, 2, true>;
+        p.policy_fn[1][1] = mpe_policy_rollout_kernel<P, 64, 2, true>;
+        p.policy_weight_floats[0][0] = PolicyShape<P, 32, 1>::kWeightFloats;
+        p.policy_weight_floats[0][1] = PolicyShape<P, 64, 1>::kWeightFloats;
+        p.policy_weight_floats[1][0] = PolicyShape<P, 32, 2>::kWeightFloats;
+        p.policy_weight_floats[1][1] = PolicyShape<P, 64, 2>::kWeightFloats;
     }
     p.smem_bytes = Shape<P>::kWarpBytes;  // per warp
     p.A = P::A; p.L = P::L; p.NS = P::NS; p.DIMC = P::DIMC; p.INFO = P::INFO; p.G = P::G;
@@ -1307,6 +1417,13 @@ static int max_warps_per_block(int smem_per_warp) {
     return fit < 1 ? 1 : (fit > kMaxWarpsPerBlock ? kMaxWarpsPerBlock : fit);
 }
 
+// dynamic shared memory of a closed-loop rollout block: the actors of all agents once, one staging slot per warp;
+// capped to what an SM offers (larger blocks are then never launched: policy_warps_per_block)
+static int policy_smem_bytes(const Program *prog, int di, int k, int wpb) {
+    const long long b = static_cast<long long>(prog->policy_weight_floats[di][k]) * 4 + static_cast<long long>(prog->smem_bytes) * wpb;
+    return b < 227 * 1024 ? static_cast<int>(b) : 227 * 1024;
+}
+
 static_assert(sizeof(mpe_desc) == 480, "mpe_desc layout is part of the ABI (mirrored by _lib.MpeDesc)");
 
 struct mpe_env {
@@ -1320,6 +1437,7 @@ struct mpe_env {
     // chunk overlaps the D2H copy of the previous one (PCIe is full duplex)
     cudaStream_t aux[2] = {nullptr, nullptr};
     cudaEvent_t ev_fork = nullptr, ev_join[2] = {nullptr, nullptr};
+    int policy2_wpb[2] = {0, 0};   // depth-2 closed-loop rollout: warps per block of most residency (0: not yet asked)
 };
 
 static thread_local char g_cuda_err[256] = "";
@@ -1374,10 +1492,14 @@ extern "C" int mpe_create(const mpe_desc *desc, int64_t n_env, int device, mpe_h
         if (prog->pipe_fn)
             CUDA_TRY(cudaFuncSetAttribute(prog->pipe_fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           prog->pipe_smem * max_warps_per_block(prog->pipe_smem)));
+        for (int dk = 0; dk < 4; ++dk)
+            if (prog->policy_fn[dk >> 1][dk & 1])
+                CUDA_TRY(cudaFuncSetAttribute(prog->policy_fn[dk >> 1][dk & 1], cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                              policy_smem_bytes(prog, dk >> 1, dk & 1, dk < 2 ? kPolicyMaxWarps<1> : kPolicyMaxWarps<2>)));
         for (int k = 0; k < 2; ++k)
-            if (prog->policy_fn[k])
-                CUDA_TRY(cudaFuncSetAttribute(prog->policy_fn[k], cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                              prog->policy_weight_floats[k] * 4 + prog->smem_bytes * 4));
+            if (prog->policy_plain_fn[k])
+                CUDA_TRY(cudaFuncSetAttribute(prog->policy_plain_fn[k], cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                              policy_smem_bytes(prog, 0, k, kPolicyMaxWarps<1>)));
         if (prog->rollout_fn)
             CUDA_TRY(cudaFuncSetAttribute(prog->rollout_fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           prog->rollout_smem * max_warps_per_block(prog->rollout_smem)));
@@ -1780,29 +1902,67 @@ extern "C" int mpe_rollout(mpe_handle h, void *pv, const void *lm, float *comm, 
     return MPE_OK;
 }
 
-extern "C" int mpe_rollout_policy(mpe_handle h, void *pv, const void *lm, float *comm, const int32_t *goal,
-                                  const float *const *w1_n, const float *const *b1_n, const float *const *w2_n,
-                                  const float *const *b2_n, int32_t hidden, int32_t n_steps, float *const *obs_n,
-                                  float *rew_sum, float *rew_steps, float *const *act_record_n, uint8_t *done,
-                                  uint32_t flags, void *stream) {
+// Depth 1 keeps its original block sizes.  Depth 2 stages 70-92 KB of weights per block (H = 64), so one-warp blocks
+// would leave an SM 2-3 warps: it takes the block size of 1-8 warps with the most resident warps per SM (registers and
+// shared memory, from the occupancy calculator; the smaller on ties), and small batches shrink it until every SM has a
+// block.
+static int policy_warps_per_block(mpe_handle h, int di, int k, int64_t warps) {
+    if (di == 0) return warps <= 148 * 16 ? 1 : (warps <= 148 * 64 ? 2 : 4);
+    int &best = h->policy2_wpb[k];
+    if (best == 0) {
+        int most = 0;
+        best = 1;
+        for (int wpb = 1; wpb <= kPolicyMaxWarps<2>; ++wpb) {
+            const long long smem = static_cast<long long>(h->prog->policy_weight_floats[di][k]) * 4 +
+                                   static_cast<long long>(h->prog->smem_bytes) * wpb;
+            if (smem > 227 * 1024) break;
+            int blocks = 0;
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, h->prog->policy_fn[di][k], 32 * wpb,
+                                                              static_cast<size_t>(smem)) != cudaSuccess)
+                break;
+            if (blocks * wpb > most) { most = blocks * wpb; best = wpb; }
+        }
+    }
+    int wpb = best;
+    if (warps < 148LL * wpb) wpb = warps >= 148 ? static_cast<int>(warps / 148) : 1;
+    return wpb;
+}
+
+extern "C" int mpe_collect(mpe_handle h, void *pv, const void *lm, float *comm, const int32_t *goal, int32_t depth,
+                           int32_t hidden, const float *const *w1_n, const float *const *b1_n, const float *const *w2_n,
+                           const float *const *b2_n, const float *const *w3_n, const float *const *b3_n, int32_t n_steps,
+                           uint64_t sample_seed, uint32_t sample_step, uint64_t world_offset, float *const *obs_n,
+                           float *rew_sum, float *rew_steps, float *const *act_record_n, float *const *obs_record_n,
+                           uint8_t *done, uint32_t flags, void *stream) {
     if (!h || n_steps < 0 || !w1_n || !b1_n || !w2_n || !b2_n) return MPE_ERR_BAD_ARG;
-    if (h->device < 0) return MPE_ERR_NO_DEVICE;
-    const int k = hidden == 32 ? 0 : (hidden == 64 ? 1 : -1);
-    if (k < 0 || h->prog->scenario == MPE_SCN_CUSTOM || h->prog->policy_fn[k] == nullptr) return MPE_ERR_UNSUPPORTED;
-    if (flags & (MPE_FLAG_DISCRETE_ACTION_INPUT | MPE_FLAG_FORCE_DISCRETE_ACTION)) return MPE_ERR_UNSUPPORTED;
+    if ((depth != 1 && depth != 2) || (hidden != 32 && hidden != 64)) return MPE_ERR_BAD_ARG;
+    if ((depth == 2) != (w3_n != nullptr) || (depth == 2) != (b3_n != nullptr)) return MPE_ERR_BAD_ARG;
+    if (static_cast<uint64_t>(sample_step) + static_cast<uint64_t>(n_steps) > (1ull << 32)) return MPE_ERR_BAD_ARG;
     if (rew_steps != nullptr && !ok4(rew_steps)) return MPE_ERR_BAD_ARG;
-    NvtxRange range("mpe_rollout_policy");
+    const int A = h->prog->A;
+    for (int i = 0; i < A; ++i) {
+        if (!ok16(w1_n[i]) || !ok16(b1_n[i]) || !ok16(w2_n[i]) || !ok4(b2_n[i])) return MPE_ERR_BAD_ARG;
+        if (depth == 2 && (!ok16(w3_n[i]) || !ok4(b3_n[i]))) return MPE_ERR_BAD_ARG;
+        if (act_record_n && act_record_n[i] != nullptr && !ok4(act_record_n[i])) return MPE_ERR_BAD_ARG;
+        if (obs_record_n && !ok16(obs_record_n[i])) return MPE_ERR_BAD_ARG;
+    }
+    if (h->device < 0) return MPE_ERR_NO_DEVICE;
+    const int di = depth - 1, k = hidden == 32 ? 0 : 1;
+    if (h->prog->scenario == MPE_SCN_CUSTOM || h->prog->policy_fn[di][k] == nullptr) return MPE_ERR_UNSUPPORTED;
+    if (flags & (MPE_FLAG_DISCRETE_ACTION_INPUT | MPE_FLAG_FORCE_DISCRETE_ACTION)) return MPE_ERR_UNSUPPORTED;
+    NvtxRange range("mpe_collect");
     PolicyArgs pa{};
     StepArgs &a = pa.s;
     int r = fill_state(h, a, pv, lm, comm, goal);
     if (r) return r;
     r = fill_outputs(h, a, obs_n, rew_sum, done, nullptr);
     if (r) return r;
-    for (int i = 0; i < h->prog->A; ++i) {
-        if (!ok16(w1_n[i]) || !ok16(b1_n[i]) || !ok16(w2_n[i]) || !ok4(b2_n[i])) return MPE_ERR_BAD_ARG;
+    for (int i = 0; i < A; ++i) {
         pa.w1[i] = w1_n[i]; pa.b1[i] = b1_n[i]; pa.w2[i] = w2_n[i]; pa.b2[i] = b2_n[i];
+        pa.w3[i] = depth == 2 ? w3_n[i] : nullptr;
+        pa.b3[i] = depth == 2 ? b3_n[i] : nullptr;
         pa.act_rec[i] = act_record_n ? act_record_n[i] : nullptr;
-        if (pa.act_rec[i] != nullptr && !ok4(pa.act_rec[i])) return MPE_ERR_BAD_ARG;
+        pa.obs_rec[i] = obs_record_n ? obs_record_n[i] : nullptr;
     }
     a.info = nullptr;
     a.flags = flags;
@@ -1812,21 +1972,42 @@ extern "C" int mpe_rollout_policy(mpe_handle h, void *pv, const void *lm, float 
     a.count = h->n;
     pa.T = n_steps;
     pa.rew_steps = rew_steps;
-    const int64_t warps = (h->n + 31) / 32;
-    const int wpb = warps <= 148 * 16 ? 1 : (warps <= 148 * 64 ? 2 : 4);
-    const int64_t blocks = (warps + wpb - 1) / wpb;
-    if (blocks > 0x7fffffffLL) return MPE_ERR_BAD_ARG;
+    pa.sample_key = make_uint2(static_cast<uint32_t>(sample_seed), static_cast<uint32_t>(sample_seed >> 32));
+    pa.world_offset = world_offset;
+    pa.sample_step = sample_step;
     int prev = 0;
     CUDA_TRY(cudaGetDevice(&prev));
     if (prev != h->device) CUDA_TRY(cudaSetDevice(h->device));
-    void *params[] = {&pa};
-    const size_t smem = static_cast<size_t>(h->prog->policy_weight_floats[k]) * 4 + static_cast<size_t>(h->prog->smem_bytes) * wpb;
-    cudaError_t e = cudaLaunchKernel(reinterpret_cast<const void *>(h->prog->policy_fn[k]), dim3(static_cast<unsigned>(blocks)),
-                                     dim3(32 * wpb), params, smem, static_cast<cudaStream_t>(stream));
+    const int64_t warps = (h->n + 31) / 32;
+    const int wpb = policy_warps_per_block(h, di, k, warps);
+    const int64_t blocks = (warps + wpb - 1) / wpb;
+    cudaError_t e = cudaErrorInvalidValue;
+    if (blocks <= 0x7fffffffLL) {
+        void *params[] = {&pa};
+        const bool plain = depth == 1 && !(flags & MPE_FLAG_SAMPLE_ACTIONS) && obs_record_n == nullptr;
+        e = cudaLaunchKernel(reinterpret_cast<const void *>(plain ? h->prog->policy_plain_fn[k] : h->prog->policy_fn[di][k]),
+                             dim3(static_cast<unsigned>(blocks)),
+                             dim3(32 * wpb), params, static_cast<size_t>(policy_smem_bytes(h->prog, di, k, wpb)),
+                             static_cast<cudaStream_t>(stream));
+    }
     if (prev != h->device) cudaSetDevice(prev);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaLaunchKernel(rollout_policy)");
+    if (blocks > 0x7fffffffLL) return MPE_ERR_BAD_ARG;
+    if (e != cudaSuccess) return cuda_fail(e, "cudaLaunchKernel(collect)");
     __atomic_add_fetch(&g_launches, 1, __ATOMIC_RELAXED);
     return MPE_OK;
+}
+
+extern "C" int mpe_rollout_policy(mpe_handle h, void *pv, const void *lm, float *comm, const int32_t *goal,
+                                  const float *const *w1_n, const float *const *b1_n, const float *const *w2_n,
+                                  const float *const *b2_n, int32_t hidden, int32_t n_steps, float *const *obs_n,
+                                  float *rew_sum, float *rew_steps, float *const *act_record_n, uint8_t *done,
+                                  uint32_t flags, void *stream) {
+    if (!h || n_steps < 0 || !w1_n || !b1_n || !w2_n || !b2_n) return MPE_ERR_BAD_ARG;
+    if (h->device < 0) return MPE_ERR_NO_DEVICE;
+    const int k = hidden == 32 ? 0 : (hidden == 64 ? 1 : -1);
+    if (k < 0 || h->prog->scenario == MPE_SCN_CUSTOM || h->prog->policy_fn[0][k] == nullptr) return MPE_ERR_UNSUPPORTED;
+    return mpe_collect(h, pv, lm, comm, goal, 1, hidden, w1_n, b1_n, w2_n, b2_n, nullptr, nullptr, n_steps, 0, 0, 0,
+                       obs_n, rew_sum, rew_steps, act_record_n, nullptr, done, flags & ~MPE_FLAG_SAMPLE_ACTIONS, stream);
 }
 
 // adjacent (dst, src, bytes) copies with equal small gaps on both sides are issued as one DMA

@@ -240,15 +240,26 @@ class MultiAgentEnv(_Env):
             return obs_n, reward_n, done_n, info_n, rew_steps
         return obs_n, reward_n, done_n, info_n
 
-    def rollout_policy(self, policies, n_steps, record_actions=False, per_step_rewards=False):
-        """T closed-loop steps in ONE kernel launch with the actors inside the kernel (mpe_rollout_policy): agent i acts
-        with softmax(W2_i relu(W1_i obs_i + b1_i) + b2_i).  policies[i] is a `torch.nn.Sequential(Linear(obs_dim_i, H),
-        ReLU(), Linear(H, 5))` or the tuple (W1 [H, obs_dim_i], b1 [H], W2 [5, H], b2 [5]) in torch's Linear layout, H = 32
-        or 64.  Returns (obs_n, reward_sum_n, done_n, info_n, extras) for the state after the last step; extras["actions"]
+    def rollout_policy(self, policies, n_steps, record_actions=False, per_step_rewards=False, record_observations=False,
+                       explore_seed=None, explore_step=0):
+        """T closed-loop steps in ONE kernel launch with the actors inside the kernel (mpe_collect).  policies[i] is agent
+        i's actor, H = 32 or 64, the same depth and H for every agent:
+          one hidden layer   a_i = softmax(W2_i relu(W1_i obs_i + b1_i) + b2_i): a `torch.nn.Sequential(Linear(obs_dim_i,
+              H), ReLU(), Linear(H, 5))` or the tuple (W1 [H, obs_dim_i], b1 [H], W2 [5, H], b2 [5]);
+          two hidden layers (the MADDPG actor) a_i = softmax(W3_i relu(W2_i relu(W1_i obs_i + b1_i) + b2_i) + b3_i): a
+              `torch.nn.Sequential(Linear(obs_dim_i, H), ReLU(), Linear(H, H), ReLU(), Linear(H, 5))` or the tuple
+              (W1, b1, W2 [H, H], b2 [H], W3 [5, H], b3 [5]);
+        all in torch's Linear layout.  explore_seed=None acts with softmax(logits); an int acts with MADDPG's exploration
+        sample softmax(logits - log(-log u)), u uniform in (0, 1) drawn from a Philox stream keyed by (explore_seed,
+        global world index, explore_step + t, agent): a sharded env draws what the full batch draws, and a rollout split
+        into calls with explore_step = 0, T1, T1 + T2, ... draws what one call does.
+        Returns (obs_n, reward_sum_n, done_n, info_n, extras) for the state after the last step; extras["actions"]
         (record_actions) is a list of [T, N, 5] tensors with the actions taken, extras["rewards"] (per_step_rewards) a
-        [T, n, N] tensor.  World state lives in registers for all T steps and no observation is written in between.
-        Batched CUDA mode; scenarios whose agents all move and are silent and whose program was built with the policy
-        kernel (simple, simple_spread N=3, simple_tag 3+1) -- anything else raises."""
+        [T, n, N] tensor, extras["observations"] (record_observations) a list of [T, N, obs_dim_i] tensors whose row t is
+        the observation agent i acted on at step t -- with the final obs_n, the (obs, act, rew, next obs) of every step.
+        World state lives in registers for all T steps.  Batched CUDA mode; scenarios whose agents all move and are
+        silent and whose program was built with the policy kernel (simple, simple_spread N=3, simple_tag 3+1) --
+        anything else raises."""
         import torch
         world = self.world
         if not world.batched:
@@ -259,35 +270,34 @@ class MultiAgentEnv(_Env):
             raise ValueError("expected %d policies, got %d" % (self.n, len(policies)))
         nw = world.bind()
         N, T = nw.n_env, int(n_steps)
-        keep, hidden = [], None
-        ptrs = ([], [], [], [])
-        for i, pol in enumerate(policies):
-            if isinstance(pol, torch.nn.Module):
-                lin = [m for m in pol.modules() if isinstance(m, torch.nn.Linear)]
-                if len(lin) != 2:
-                    raise ValueError("policy %d must be Linear -> ReLU -> Linear" % i)
-                pol = (lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias)
-            W1, b1, W2, b2 = [t.detach().to(device=nw.device, dtype=torch.float32) for t in pol]
-            H = int(W1.shape[0])
-            if hidden is None:
-                hidden = H
-            if H != hidden or tuple(W1.shape) != (H, nw.obs_dims[i]) or tuple(b1.shape) != (H,) or \
-                    tuple(W2.shape) != (5, H) or tuple(b2.shape) != (5,):
-                raise ValueError("policy %d: expected W1 [%d, %d], b1 [%d], W2 [5, %d], b2 [5]"
-                                 % (i, hidden, nw.obs_dims[i], hidden, hidden))
-            parts = (W1.t().contiguous(), b1.contiguous(), W2.contiguous(), b2.contiguous())   # W1 input-major for the kernel
-            keep.append(parts)
-            for lst, t in zip(ptrs, parts):
-                lst.append(t.data_ptr())
+        flags = self._flags()
+        if explore_seed is not None:
+            explore_seed, explore_step = int(explore_seed), int(explore_step)
+            if not 0 <= explore_seed < 2 ** 64:
+                raise ValueError("explore_seed must be in [0, 2**64), got %d" % explore_seed)
+            if explore_step < 0 or explore_step + T >= 2 ** 32:
+                raise ValueError("explore_step + n_steps must stay below 2**32 (the step counter of the noise stream)")
+            flags |= _lib.FLAG_SAMPLE_ACTIONS
+        depth, hidden, params = actor_parameters(policies, nw.obs_dims)
+        keep = []
+        for W in params:
+            W = [t.detach().to(device=nw.device, dtype=torch.float32) for t in W]
+            W[0] = W[0].t()                      # W1 input-major for the kernel
+            keep.append([t.contiguous() for t in W])
+        ptrs = [_lib.ptr_array([W[k].data_ptr() for W in keep]) if k < len(keep[0]) else None for k in range(6)]
         out = nw.out if self.reuse_buffers else nw.new_outputs()
         rew_steps = torch.empty((T, self.n, N), dtype=torch.float32, device=nw.device) if per_step_rewards else None
         actions = [torch.empty((T, N, 5), dtype=torch.float32, device=nw.device) for _ in range(self.n)] if record_actions else None
-        nw.rollout_policy(*[_lib.ptr_array(p) for p in ptrs], hidden, T, out, self._flags(), rew_steps,
-                          _lib.ptr_array([a.data_ptr() for a in actions]) if actions is not None else None)
+        observations = [torch.empty((T, N, od), dtype=torch.float32, device=nw.device)
+                        for od in nw.obs_dims] if record_observations else None
+        nw.collect(depth, hidden, ptrs, T, out, flags, explore_seed or 0, explore_step if explore_seed is not None else 0,
+                   rew_steps, _lib.ptr_array([a.data_ptr() for a in actions]) if actions is not None else None,
+                   _lib.ptr_array([o.data_ptr() for o in observations]) if observations is not None else None)
         self._last_out = out
         world._obs_valid = False
         info_n = {'n': [{} for _ in range(self.n)]}
-        return list(out.obs), list(out.rew_list), list(out.done_list), info_n, {"actions": actions, "rewards": rew_steps}
+        return list(out.obs), list(out.rew_list), list(out.done_list), info_n, \
+            {"actions": actions, "rewards": rew_steps, "observations": observations}
 
     # ---- user scenarios: native _set_action + World.step, callbacks in the user's torch code -------
     def _step_custom(self, action_n, nw, flags):
@@ -544,3 +554,39 @@ class MultiAgentEnv(_Env):
             center = (0.0, 0.0) if self.shared_viewer else tuple(pv[i, 0:2])
             results.append(draw_world(pos, sizes, colors, alphas, center=center))
         return results
+
+
+def actor_parameters(policies, obs_dims):
+    """(depth, H, [per-agent weight tuples in torch's Linear layout]) of the actors MultiAgentEnv.rollout_policy runs:
+    depth 1 -- a module holding exactly two Linear layers (Linear -> ReLU -> Linear) or (W1, b1, W2, b2); depth 2 -- a
+    `Sequential(Linear, ReLU, Linear, ReLU, Linear)` or (W1, b1, W2, b2, W3, b3).  Every agent must have the same depth
+    and H, and the shapes must fit its observation; anything else raises ValueError.  Works on tensors of any device."""
+    import torch
+    depth = hidden = None
+    params = []
+    for i, pol in enumerate(policies):
+        if isinstance(pol, torch.nn.Module):
+            lin = [m for m in pol.modules() if isinstance(m, torch.nn.Linear)]
+            if len(lin) == 2:
+                pol = (lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias)
+            elif len(lin) == 3:
+                kinds = [type(m) for m in pol.children()] if isinstance(pol, torch.nn.Sequential) else []
+                if kinds != [torch.nn.Linear, torch.nn.ReLU, torch.nn.Linear, torch.nn.ReLU, torch.nn.Linear]:
+                    raise ValueError("policy %d must be Linear -> ReLU -> Linear -> ReLU -> Linear" % i)
+                pol = tuple(t for m in lin for t in (m.weight, m.bias))
+            else:
+                raise ValueError("policy %d must be Linear -> ReLU -> Linear" % i)
+        pol = tuple(pol)
+        if len(pol) not in (4, 6):
+            raise ValueError("policy %d: expected (W1, b1, W2, b2) or (W1, b1, W2, b2, W3, b3), got %d tensors" % (i, len(pol)))
+        d, H = len(pol) // 2 - 1, int(pol[0].shape[0])
+        if depth is None:
+            depth, hidden = d, H
+        if d != depth:
+            raise ValueError("policy %d has %d hidden layers, policy 0 has %d: all actors must have the same depth" % (i, d, depth))
+        want = [(hidden, obs_dims[i]), (hidden,)] + ([(5, hidden), (5,)] if depth == 1 else
+                                                      [(hidden, hidden), (hidden,), (5, hidden), (5,)])
+        if [tuple(t.shape) for t in pol] != want:
+            raise ValueError("policy %d: expected shapes %s, got %s" % (i, want, [tuple(t.shape) for t in pol]))
+        params.append(pol)
+    return depth, hidden, params

@@ -273,6 +273,20 @@ class NativeWorld(ShapeHandle):
                                           out.done_ptr, flags, self._stream()), "mpe_rollout_policy")
         return out
 
+    def collect(self, depth, hidden, weight_ptrs, n_steps, out=None, flags=0, sample_seed=0, sample_step=0, rew_steps=None,
+                act_rec_ptrs=None, obs_rec_ptrs=None):
+        """n_steps closed-loop steps in ONE launch with one- or two-hidden-layer actors inside the kernel (mpe_collect).
+        weight_ptrs: the pointer arrays (w1, b1, w2, b2, w3, b3), one device pointer per agent (w3, b3 None at depth 1).
+        The exploration noise is keyed by this shard's global world indices (world_offset), so a sharded batch draws
+        what the whole batch draws."""
+        out = out or self.out
+        pv, lm, comm, goal = self._state_ptrs()
+        check(self.lib.mpe_collect(self.handle, pv, lm, comm, goal, int(depth), int(hidden), *weight_ptrs, int(n_steps),
+                                   int(sample_seed), int(sample_step), self.world_offset, out.obs_ptrs, out.rew_ptr,
+                                   rew_steps.data_ptr() if rew_steps is not None else None, act_rec_ptrs, obs_rec_ptrs,
+                                   out.done_ptr, flags, self._stream()), "mpe_collect")
+        return out
+
     # ---- host callers (what the reference's callers hold: NumPy arrays) -----------------------
     def host_staging(self):
         if self._host is None:
