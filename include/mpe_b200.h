@@ -199,8 +199,8 @@ MPE_API int mpe_rollout(mpe_handle h, void *agent_pv_dev, const void *lm_p_dev, 
  * hidden = 32 or 64.  World state stays in registers, observations are never written between steps.  Outputs as
  * mpe_rollout; act_record_n (NULL or per agent float [n_steps][n_env][5]) receives the actions taken -- feeding them to
  * mpe_rollout / mpe_step reproduces state, observations and reward sums bit for bit.  Only for scenarios whose agents
- * all move and are silent and for which the program was built (the BASELINE.json worlds simple, simple_spread N = 3,
- * simple_tag 3 + 1); otherwise MPE_ERR_UNSUPPORTED. */
+ * all move and are silent and for which the program was built (simple, simple_spread N = 3, simple_tag 3 + 1,
+ * simple_adversary 1 + 2, simple_push); otherwise, speaking or immovable agents included, MPE_ERR_UNSUPPORTED. */
 MPE_API int mpe_rollout_policy(mpe_handle h, void *agent_pv_dev, const void *lm_p_dev, float *comm_dev,
                                const int32_t *goal_dev, const float *const *w1_n, const float *const *b1_n,
                                const float *const *w2_n, const float *const *b2_n, int32_t hidden, int32_t n_steps,
@@ -210,27 +210,36 @@ MPE_API int mpe_rollout_policy(mpe_handle h, void *agent_pv_dev, const void *lm_
 /* Training experience in ONE launch: the closed loop of mpe_rollout_policy, with a one- or two-hidden-layer actor,
  * optional exploration noise and a record of every step's observations -- everything a replay buffer needs:
  * (obs_record[t], act_record[t], rew_steps[t], obs_record[t + 1]), with obs_n_dev holding the observation after the
- * last step.
- *   depth 1:  a_i = softmax(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i)                          (obs_dim_i -> H -> 5)
- *   depth 2:  a_i = softmax(W3_i . relu(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i) + b3_i)      (obs_dim_i -> H -> H -> 5,
- *             the MADDPG actor: fc 64 relu, fc 64 relu, fc 5)
+ * last step.  Agent i's actor has act_dim_i = mpe_act_dim(h, i) outputs:
+ *   depth 1:  logits_i = W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i                          (obs_dim_i -> H -> act_dim_i)
+ *   depth 2:  logits_i = W3_i . relu(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i) + b3_i      (obs_dim_i -> H -> H ->
+ *             act_dim_i, the MADDPG actor: fc 64 relu, fc 64 relu, fc act_dim_i)
+ * The logits are the heads of the reference's action space (environment.py:58-64): 5 movement logits if the agent
+ * moves, then dim_c communication logits if it speaks.  Each head gets its own max-subtracted softmax; the action is
+ * [softmax(movement) | softmax(comm)], the comm head's probabilities becoming the agent's utterance (action.c) once
+ * every agent has acted on the current state, as in mpe_step.
  * hidden = H = 32 or 64.  Weights, all 16-byte aligned except b2 / b3 (4-byte):
  *   w1_n[i] float [obs_dim_i][H] (input-major, W1^T of a torch Linear(obs_dim_i, H)), b1_n[i] [H];
- *   depth 1: w2_n[i] [5][H], b2_n[i] [5], w3_n = b3_n = NULL;
- *   depth 2: w2_n[i] [H][H] (torch Linear(H, H).weight), b2_n[i] [H], w3_n[i] [5][H], b3_n[i] [5].
- * Every unit sums bias + inputs in ascending input order with FMAs.
- * flags: MPE_FLAG_SHARED_REWARD as for mpe_step; MPE_FLAG_SAMPLE_ACTIONS replaces softmax(logits) by the exploration
- * sample softmax(logits - log(-log u)), u = (2 (bits >> 9) + 1) 2^-24 from Philox4x32-10 with key (sample_seed lo, hi)
- * and counter (w lo, w hi, sample_step + t, 0x40000000 | agent << 1 | block), w = world_offset + world index, blocks 0
- * and 1 giving words 0-3 and 4 for the five logits.  Draws depend on the global world index and the global step only,
- * so a sharded batch or a rollout split into several calls draws exactly what one call over the whole batch draws.
- * Records (NULL, or per agent): act_record_n[i] float [n_steps][n_env][5], the actions taken (sampled ones when
+ *   depth 1: w2_n[i] [act_dim_i][H], b2_n[i] [act_dim_i], w3_n = b3_n = NULL;
+ *   depth 2: w2_n[i] [H][H] (torch Linear(H, H).weight), b2_n[i] [H], w3_n[i] [act_dim_i][H], b3_n[i] [act_dim_i].
+ * Every unit sums bias + inputs in ascending input order with FMAs.  comm_dev (the speakers' utterances) is read
+ * before the first step and written after the last; it is required when the scenario has speakers.
+ * flags: MPE_FLAG_SHARED_REWARD as for mpe_step; MPE_FLAG_SAMPLE_ACTIONS replaces each head's softmax(logits) by the
+ * exploration sample softmax(logits - log(-log u)), u = (2 (bits >> 9) + 1) 2^-24 from Philox4x32-10 with key
+ * (sample_seed lo, hi) and counter (w lo, w hi, sample_step + t, tag), w = world_offset + world index:
+ *   movement logit c < 5: tag 0x40000000 | agent << 1 | block, blocks 0 and 1 giving words 0-3 and 4;
+ *   comm logit q < dim_c: word q & 3 of block q >> 2 with tag 0x40000100 | agent << 2 | block.
+ * These counters are disjoint from each other and from mpe_reset's (small block numbers, 0x80000000 in word 3).  Draws
+ * depend on the global world index and the global step only, so a sharded batch or a rollout split into several calls
+ * draws exactly what one call over the whole batch draws.
+ * Records (NULL, or per agent): act_record_n[i] float [n_steps][n_env][act_dim_i], the actions taken (sampled ones when
  * sampling); obs_record_n[i] float [n_steps][n_env][obs_dim_i] (16-byte aligned, all agents or none), row t = the
  * observation agent i acted on at step t (row 0 = the state before the call).  Feeding act_record_n to mpe_step
- * reproduces state, observations and rewards bit for bit.  Outputs otherwise as mpe_rollout_policy.
+ * reproduces state, utterances, observations and rewards bit for bit.  Outputs otherwise as mpe_rollout_policy.
+ * For scenarios whose agents all move and are silent nothing differs from a 5-wide actor.
  * Errors: MPE_ERR_BAD_ARG for NULL / misaligned pointers, depth not 1 or 2, hidden not 32 or 64, n_steps < 0 or
  * sample_step + n_steps > 2^32; MPE_ERR_NO_DEVICE for a device-less handle; MPE_ERR_UNSUPPORTED for a scenario
- * without the kernel (as mpe_rollout_policy) or MPE_FLAG_FORCE_DISCRETE_ACTION / MPE_FLAG_DISCRETE_ACTION_INPUT. */
+ * without the kernel (mpe_collect_supported) or MPE_FLAG_FORCE_DISCRETE_ACTION / MPE_FLAG_DISCRETE_ACTION_INPUT. */
 MPE_API int mpe_collect(mpe_handle h, void *agent_pv_dev, const void *lm_p_dev, float *comm_dev, const int32_t *goal_dev,
                         int32_t depth, int32_t hidden,
                         const float *const *w1_n, const float *const *b1_n,
@@ -240,6 +249,12 @@ MPE_API int mpe_collect(mpe_handle h, void *agent_pv_dev, const void *lm_p_dev, 
                         float *const *obs_n_dev, float *rew_sum_dev, float *rew_steps_dev,
                         float *const *act_record_n, float *const *obs_record_n, uint8_t *done_dev,
                         uint32_t flags, void *stream);
+
+/* Is mpe_collect built for this handle's scenario at this depth and hidden width?  MPE_OK; MPE_ERR_UNSUPPORTED (built
+ * for simple, simple_spread N = 3, simple_tag 3 + 1, simple_adversary 1 + 2, simple_push, simple_speaker_listener,
+ * simple_reference and simple_crypto; not for user scenarios or other entity counts); MPE_ERR_BAD_ARG for a NULL handle,
+ * depth not 1 or 2 or hidden not 32 or 64.  Needs no device: answers for shape-only handles as well. */
+MPE_API int mpe_collect_supported(mpe_handle h, int32_t depth, int32_t hidden);
 
 /* Same step for a caller that holds HOST buffers (what the reference's callers hold):
  * act_n_host[i] -> (async H2D into act_n_dev[i]) -> mpe_step -> (async D2H) obs_n_host[i],

@@ -92,6 +92,7 @@ _SIGNATURES = {
     "mpe_collect": (ctypes.c_int, [_P, _P, _P, _P, _P, ctypes.c_int32, ctypes.c_int32, _PP, _PP, _PP, _PP, _PP, _PP,
                                    ctypes.c_int32, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint64, _PP, _P, _P, _PP, _PP,
                                    _P, ctypes.c_uint32, _P]),
+    "mpe_collect_supported": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32]),
     "mpe_step_host": (ctypes.c_int, [_P, _P, _P, _P, _P, _PP, _PP, _PP, _P, _P, _P, _PP, _P, _P, _P,
                                      ctypes.c_uint32, _P]),
     "mpe_strerror": (ctypes.c_char_p, [ctypes.c_int]),

@@ -793,41 +793,48 @@ __global__ void __launch_bounds__(MPE_BOUND_THREADS, MPE_MIN_BLOCKS) mpe_rollout
 // ---- K-step CLOSED-LOOP rollout with an in-kernel policy (SURVEY.md 8(f) rank 3, the persistent form with a device-
 // resident policy; VERDICT r1 item 9) -------------------------------------------------------------------------------
 // T consecutive MultiAgentEnv.step calls in ONE launch where every agent's action is produced inside the kernel by its
-// own perceptron.  DEPTH 1:  a_i = softmax(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i)  (obs_dim_i -> H -> 5 movement
-// probabilities); DEPTH 2, the MADDPG actor:  a_i = softmax(W3_i . relu(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i) + b3_i)
-// (obs_dim_i -> H -> H -> 5).  A world's state lives in registers for all T steps; an agent's observation is produced
-// straight into registers, pushed through the perceptron (weights of all agents sit in shared memory once per block,
-// read as broadcast LDS.128), decoded and integrated.  Per step NOTHING is read from HBM and only the optional records
-// (rewards, actions, observations) are written; observations are always written for the final state.
+// own perceptron.  DEPTH 1:  logits_i = W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i  (obs_dim_i -> H -> act_dim_i);
+// DEPTH 2, the MADDPG actor:  logits_i = W3_i . relu(W2_i . relu(W1_i^T . obs_i + b1_i) + b2_i) + b3_i
+// (obs_dim_i -> H -> H -> act_dim_i).  The logits split into the heads of the reference's action space
+// (environment.py:58-64, MADDPG samples each head on its own): 5 movement logits if the agent moves, then dim_c
+// communication logits if it speaks; each head gets its own softmax.  A world's state lives in registers for all T
+// steps; an agent's observation is produced straight into registers, pushed through the perceptron (weights of all
+// agents sit in shared memory once per block, read as broadcast LDS.128), decoded and integrated.  Per step NOTHING is
+// read from HBM and only the optional records (rewards, actions, observations) are written; observations are always
+// written for the final state.
 // With MPE_FLAG_SAMPLE_ACTIONS the action is MADDPG's exploration sample softmax(logits + g), g = -log(-log u) Gumbel
-// noise from a Philox stream keyed by (seed, global world, step, agent), so trajectories do not depend on sharding.
-// Scenarios whose agents all move and are silent (simple_spread, simple_tag, ...).  The physics / reward / observation
-// arithmetic is the fused step's: feeding the recorded actions to T fused steps reproduces the final state, the
-// observations and the reward sums bit for bit; the perceptron matches a float64 evaluation to ~1e-6 (tests).
+// noise from a Philox stream keyed by (seed, global world, step, agent, logit), so trajectories do not depend on
+// sharding.  The physics / reward / observation arithmetic is the fused step's: feeding the recorded actions to T fused
+// steps reproduces the final state, the communication state, the observations and the reward sums bit for bit; the
+// perceptron matches a float64 evaluation to ~1e-6 (tests).
 struct PolicyArgs {
     StepArgs s;
     int32_t T;
     float *rew_steps;               // [T][A][n] or null
-    float *act_rec[kMaxA];          // [T][n][5] per agent, or null
+    float *act_rec[kMaxA];          // [T][n][act_dim_i] per agent, or null
     float *obs_rec[kMaxA];          // [T][n][obs_dim_i] per agent (row t: the observation acted on at step t), or all null
     const float *w1[kMaxA];         // [obs_dim_i][H]  (input-major: W1^T of a torch Linear(obs_dim_i, H))
     const float *b1[kMaxA];         // [H]
-    const float *w2[kMaxA];         // depth 1: [5][H] (torch Linear(H, 5).weight); depth 2: [H][H] (Linear(H, H).weight)
-    const float *b2[kMaxA];         // depth 1: [5]; depth 2: [H]
-    const float *w3[kMaxA];         // depth 2: [5][H] (torch Linear(H, 5).weight); depth 1: unused
-    const float *b3[kMaxA];         // depth 2: [5]
+    const float *w2[kMaxA];         // depth 1: [act_dim_i][H] (torch Linear(H, act_dim_i).weight); depth 2: [H][H]
+    const float *b2[kMaxA];         // depth 1: [act_dim_i]; depth 2: [H]
+    const float *w3[kMaxA];         // depth 2: [act_dim_i][H] (torch Linear(H, act_dim_i).weight); depth 1: unused
+    const float *b3[kMaxA];         // depth 2: [act_dim_i]
     uint2 sample_key;               // Philox key of the exploration noise (MPE_FLAG_SAMPLE_ACTIONS)
     uint64_t world_offset;          // global index of world 0 of this batch
     uint32_t sample_step;           // global step index of step 0 of this launch
 };
 
-// shared-memory image of one agent's actor (floats, every part 16-byte aligned):
-//   depth 1: [W1: OD x H][b1: H][W2: 5 x H][b2: 5, padded to 8]
-//   depth 2: [W1: OD x H][b1: H][W2: H x H][b2: H][W3: H x 8, input-major, outputs 5..7 zero][b3: 5, padded to 8]
+__host__ __device__ constexpr int pad4(int x) { return (x + 3) & ~3; }
+__host__ __device__ constexpr int ilog2(int x) { return x > 1 ? 1 + ilog2(x >> 1) : 0; }
+
+// shared-memory image of one agent's actor (floats, every part 16-byte aligned), AD = act_dim_i, AP = pad4(AD):
+//   depth 1: [W1: OD x H][b1: H][W2: AD x H][b2: AD, padded to AP]
+//   depth 2: [W1: OD x H][b1: H][W2: H x H][b2: H][W3: H x AP, input-major, outputs AD..AP-1 zero][b3: AD, padded to AP]
 template <class P, int H, int DEPTH>
 struct PolicyShape {
     __host__ __device__ static constexpr int agent_floats(int i) {
-        return P::obs_dim(i) * H + H + (DEPTH == 1 ? 5 * H + 8 : H * H + H + 8 * H + 8);
+        const int AD = P::act_dim(i), AP = pad4(AD);
+        return P::obs_dim(i) * H + H + (DEPTH == 1 ? AD * H + AP : H * H + H + AP * H + AP);
     }
     __host__ __device__ static constexpr int agent_off(int i) { int s = 0; for (int j = 0; j < i; ++j) s += agent_floats(j); return s; }
     static constexpr int kWeightFloats = (agent_off(P::A) + 3) & ~3;
@@ -844,19 +851,49 @@ struct RegWriter {
 };
 
 // Philox counter word 3 of the exploration noise: bit 30 set keeps it apart from the reset stream (small block numbers
-// and 0x80000000); two blocks per (world, step, agent), 5 of their 8 words used
+// and 0x80000000).  Movement logits: two blocks per (world, step, agent), 5 of their 8 words used.  Communication
+// logit q: word q & 3 of block q >> 2 under 0x40000100 | agent << 2 | block (dim_c <= 16), which no movement tag
+// (at most 0x4000000f) reaches.
 __host__ __device__ constexpr uint32_t sample_tag(int agent, int block) { return 0x40000000u | (static_cast<uint32_t>(agent) << 1) | block; }
+__host__ __device__ constexpr uint32_t comm_sample_tag(int agent, int block) {
+    return 0x40000100u | (static_cast<uint32_t>(agent) << 2) | block;
+}
 
-// one agent of the in-kernel policy: observation -> registers -> perceptron -> (+ Gumbel noise) -> softmax -> decoded
-// (u.x, u.y).  A plain force-inlined function with unrolled loops (not a lambda: arrays captured by reference by a lambda
-// that the compiler declines to inline end up in local memory).  W = the agent's PolicyShape image in shared memory.
+// (2 k + 1) 2^-24, k < 2^23: exact in fp32 and strictly inside (0, 1), so both logarithms of the Gumbel term are finite
+__device__ __forceinline__ float gumbel(uint32_t bits) {
+    const float u = static_cast<float>(2u * (bits >> 9) + 1u) * 5.9604644775390625e-8f;
+    return -logf(-logf(u));
+}
+
+// in-place softmax of one action head: max-subtracted, exponentials summed in ascending order
+template <int N>
+__device__ __forceinline__ void head_softmax(float *v) {
+    float m = v[0];
+#pragma unroll
+    for (int c = 1; c < N; ++c) m = fmaxf(m, v[c]);
+    float sum = 0.0f;
+#pragma unroll
+    for (int c = 0; c < N; ++c) { v[c] = expf(__fsub_rn(v[c], m)); sum = __fadd_rn(sum, v[c]); }
+#pragma unroll
+    for (int c = 0; c < N; ++c) v[c] = __fdiv_rn(v[c], sum);
+}
+
+// one agent of the in-kernel policy: observation -> registers -> perceptron -> (+ Gumbel noise) -> per-head softmax ->
+// decoded (u.x, u.y) of the movement head (zero for an immovable agent) and, for a speaker, the communication head's
+// probabilities in cact[I * dim_c ...] (action.c).  A plain force-inlined function with unrolled loops (not a lambda:
+// arrays captured by reference by a lambda that the compiler declines to inline end up in local memory).  W = the
+// agent's PolicyShape image in shared memory.
 // Summation order (fixed; the float64 tests rely on it): every unit starts from its bias and adds its inputs in
 // ascending order with FMAs -- layer 1 over j = observation index, layer 2 over j = layer-1 unit, the output layer over
 // q = last hidden unit.
-template <class P, int H, int DEPTH, int I>
+template <class P, int H, int DEPTH, int I, int NC>
 __device__ __forceinline__ float2 policy_agent(const DevDesc &d, const typename P::W &w, const float *__restrict__ W,
-                                               float *__restrict__ record, bool sample, uint2 key, uint64_t gw, uint32_t step) {
-    constexpr int OD = P::obs_dim(I);
+                                               float *__restrict__ record, bool sample, uint2 key, uint64_t gw, uint32_t step,
+                                               float (&cact)[NC]) {
+    constexpr int OD = P::obs_dim(I), AD = P::act_dim(I), AP = pad4(AD);
+    constexpr bool MOVE = P::movable(I), SPEAK = I < P::NS;
+    constexpr int C0 = MOVE ? 5 : 0;                       // first communication logit
+    static_assert(AD == C0 + (SPEAK ? P::DIMC : 0) && AD > 0 && P::DIMC <= 16, "policy rollout: action heads");
     const float *W1 = W, *B1 = W1 + OD * H, *W2 = B1 + H;
     RegWriter<OD> o;
     P::template observe<I>(d, w, o);                       // scenario.observation(agent I) -> registers
@@ -880,11 +917,11 @@ __device__ __forceinline__ float2 policy_agent(const DevDesc &d, const typename 
     }
 #pragma unroll
     for (int q = 0; q < H; ++q) h[q] = fmaxf(h[q], 0.0f);  // ReLU
-    float lg[5];
+    float lg[AD];
     if constexpr (DEPTH == 1) {
-        const float *B2 = W2 + 5 * H;
+        const float *B2 = W2 + AD * H;
 #pragma unroll
-        for (int c = 0; c < 5; ++c) {                      // logits[c] = b2[c] + sum_q h[q] * W2[c][q]  (ascending q)
+        for (int c = 0; c < AD; ++c) {                     // logits[c] = b2[c] + sum_q h[q] * W2[c][q]  (ascending q)
             float acc = B2[c];
 #pragma unroll
             for (int q = 0; q < H; q += 4) {
@@ -898,13 +935,13 @@ __device__ __forceinline__ float2 policy_agent(const DevDesc &d, const typename 
         }
     } else {
         // The second hidden layer is never materialised: unit q is computed, rectified and immediately folded into the
-        // five logits, so only h[H] and lg[5] stay live (the register profile of depth 1).  The q loop stays rolled
+        // logits, so only h[H] and lg[AD] stay live (the register profile of depth 1).  The q loop stays rolled
         // (H x H unrolled FMAs per agent would overflow the instruction cache); the j loop is unrolled because h needs
         // compile-time indices.  h2_q = relu(b2[q] + sum_j h[j] W2[q][j]) (ascending j), then
         // logits[c] = b3[c] + sum_q h2_q W3[c][q] (ascending q).
-        const float *B2 = W2 + H * H, *W3 = B2 + H, *B3 = W3 + 8 * H;
+        const float *B2 = W2 + H * H, *W3 = B2 + H, *B3 = W3 + AP * H;
 #pragma unroll
-        for (int c = 0; c < 5; ++c) lg[c] = B3[c];
+        for (int c = 0; c < AD; ++c) lg[c] = B3[c];
 #pragma unroll 1
         for (int q = 0; q < H; ++q) {
             const float *row = W2 + q * H;
@@ -918,43 +955,66 @@ __device__ __forceinline__ float2 policy_agent(const DevDesc &d, const typename 
                 acc = __fmaf_rn(h[j + 3], wv.w, acc);
             }
             acc = fmaxf(acc, 0.0f);
-            const float4 wa = *reinterpret_cast<const float4 *>(W3 + 8 * q);
-            const float4 wb = *reinterpret_cast<const float4 *>(W3 + 8 * q + 4);
-            lg[0] = __fmaf_rn(acc, wa.x, lg[0]);
-            lg[1] = __fmaf_rn(acc, wa.y, lg[1]);
-            lg[2] = __fmaf_rn(acc, wa.z, lg[2]);
-            lg[3] = __fmaf_rn(acc, wa.w, lg[3]);
-            lg[4] = __fmaf_rn(acc, wb.x, lg[4]);
+            float4 wv[AP / 4];                             // row q of W3: AP / 4 broadcast LDS.128
+            static_for<AP / 4>([&](auto vc) {              // straight-line code: an inner loop, even unrolled, changes
+                constexpr int v = decltype(vc)::value;     // how the rolled q loop is compiled
+                wv[v] = *reinterpret_cast<const float4 *>(W3 + AP * q + 4 * v);
+            });
+            static_for<AD>([&](auto cc) {
+                constexpr int c = decltype(cc)::value;
+                const float4 &u = wv[c >> 2];
+                lg[c] = __fmaf_rn(acc, (c & 3) == 0 ? u.x : (c & 3) == 1 ? u.y : (c & 3) == 2 ? u.z : u.w, lg[c]);
+            });
         }
     }
     if (sample) {   // MADDPG's exploration: softmax(logits - log(-log u)), u uniform in (0, 1)
         const uint4 ctr = make_uint4(static_cast<uint32_t>(gw), static_cast<uint32_t>(gw >> 32), step, sample_tag(I, 0));
-        const uint4 r0 = philox4x32_10(ctr, key);
-        const uint4 r1 = philox4x32_10(make_uint4(ctr.x, ctr.y, ctr.z, sample_tag(I, 1)), key);
-        const uint32_t bits[5] = {r0.x, r0.y, r0.z, r0.w, r1.x};
+        if constexpr (MOVE) {
+            const uint4 r0 = philox4x32_10(ctr, key);
+            const uint4 r1 = philox4x32_10(make_uint4(ctr.x, ctr.y, ctr.z, sample_tag(I, 1)), key);
+            const uint32_t bits[5] = {r0.x, r0.y, r0.z, r0.w, r1.x};
 #pragma unroll
-        for (int c = 0; c < 5; ++c) {
-            // (2 k + 1) 2^-24, k < 2^23: exact in fp32 and strictly inside (0, 1), so both logarithms are finite
-            const float u = static_cast<float>(2u * (bits[c] >> 9) + 1u) * 5.9604644775390625e-8f;
-            lg[c] = __fadd_rn(lg[c], -logf(-logf(u)));
+            for (int c = 0; c < 5; ++c) lg[c] = __fadd_rn(lg[c], gumbel(bits[c]));
+        }
+        if constexpr (SPEAK) {
+#pragma unroll
+            for (int b = 0; b < (P::DIMC + 3) / 4; ++b) {
+                const uint4 r = philox4x32_10(make_uint4(ctr.x, ctr.y, ctr.z, comm_sample_tag(I, b)), key);
+                const uint32_t bits[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+                for (int q = 4 * b; q < P::DIMC && q < 4 * b + 4; ++q) lg[C0 + q] = __fadd_rn(lg[C0 + q], gumbel(bits[q & 3]));
+            }
         }
     }
-    const float m = fmaxf(fmaxf(fmaxf(lg[0], lg[1]), fmaxf(lg[2], lg[3])), lg[4]);
-    float e[5], sum = 0.0f;
+    float pr[AD];                                          // per-head softmax: the action vector [movement | comm]
+    if constexpr (MOVE) {
+        const float m = fmaxf(fmaxf(fmaxf(lg[0], lg[1]), fmaxf(lg[2], lg[3])), lg[4]);
+        float e[5], sum = 0.0f;
 #pragma unroll
-    for (int c = 0; c < 5; ++c) { e[c] = expf(__fsub_rn(lg[c], m)); sum = __fadd_rn(sum, e[c]); }
-    float pr[5];
+        for (int c = 0; c < 5; ++c) { e[c] = expf(__fsub_rn(lg[c], m)); sum = __fadd_rn(sum, e[c]); }
 #pragma unroll
-    for (int c = 0; c < 5; ++c) pr[c] = __fdiv_rn(e[c], sum);                // softmax: the action vector
+        for (int c = 0; c < 5; ++c) pr[c] = __fdiv_rn(e[c], sum);
+    }
+    if constexpr (SPEAK) {
+#pragma unroll
+        for (int q = 0; q < P::DIMC; ++q) pr[C0 + q] = lg[C0 + q];
+        head_softmax<P::DIMC>(pr + C0);
+#pragma unroll
+        for (int q = 0; q < P::DIMC; ++q) cact[I * P::DIMC + q] = pr[C0 + q];   // action.c (environment.py:183-190)
+    }
     if (record != nullptr) {
 #pragma unroll
-        for (int c = 0; c < 5; ++c) record[c] = pr[c];
+        for (int c = 0; c < AD; ++c) record[c] = pr[c];
     }
-    // _set_action (environment.py:173-181), the arithmetic of decode_rows
-    float x = 0.0f, y = 0.0f;
-    x += pr[1] - pr[2];
-    y += pr[3] - pr[4];
-    return make_float2(__fmul_rn(x, d.a_sens[I]), __fmul_rn(y, d.a_sens[I]));
+    if constexpr (MOVE) {
+        // _set_action (environment.py:173-181), the arithmetic of decode_rows
+        float x = 0.0f, y = 0.0f;
+        x += pr[1] - pr[2];
+        y += pr[3] - pr[4];
+        return make_float2(__fmul_rn(x, d.a_sens[I]), __fmul_rn(y, d.a_sens[I]));
+    } else {
+        return make_float2(0.0f, 0.0f);
+    }
 }
 
 // block sizes: depth 1 as it always was (1, 2 or 4 warps); depth 2 up to 8 warps, because its weights (70-92 KB at
@@ -967,9 +1027,9 @@ constexpr int kPolicyMaxWarps = DEPTH == 1 ? 4 : 8;
 // step at 65 536 worlds (B200, 1000 W), so depth 1 keeps the plain build for plain calls.
 template <class P, int H, int DEPTH, bool EXTRAS>
 __global__ void __launch_bounds__(32 * kPolicyMaxWarps<DEPTH>) mpe_policy_rollout_kernel(const __grid_constant__ PolicyArgs pa) {
-    static_assert(P::NS == 0 && H % 4 == 0, "policy rollout: silent agents, hidden width a multiple of 4");
+    static_assert(H % 4 == 0, "policy rollout: hidden width a multiple of 4");
     static_assert(DEPTH == 1 || DEPTH == 2, "policy rollout: one or two hidden layers");
-    constexpr int A = P::A, L = P::L;
+    constexpr int A = P::A, L = P::L, NC = Shape<P>::kNC;
     using PS = PolicyShape<P, H, DEPTH>;
     const StepArgs &a = pa.s;
     extern __shared__ __align__(16) float smem[];
@@ -978,21 +1038,24 @@ __global__ void __launch_bounds__(32 * kPolicyMaxWarps<DEPTH>) mpe_policy_rollou
     // ---- all agents' weights -> shared memory, once per block ------------------------------------------------
     static_for<A>([&](auto ic) {
         constexpr int i = decltype(ic)::value;
-        constexpr int OD = P::obs_dim(i);
+        constexpr int OD = P::obs_dim(i), AD = P::act_dim(i), AP = pad4(AD);
         float *base = s_w + PS::agent_off(i);
         for (int q = threadIdx.x; q < OD * H; q += blockDim.x) base[q] = pa.w1[i][q];
         for (int q = threadIdx.x; q < H; q += blockDim.x) base[OD * H + q] = pa.b1[i][q];
         base += OD * H + H;
         if constexpr (DEPTH == 1) {
-            for (int q = threadIdx.x; q < 5 * H; q += blockDim.x) base[q] = pa.w2[i][q];
-            for (int q = threadIdx.x; q < 5; q += blockDim.x) base[5 * H + q] = pa.b2[i][q];
+            for (int q = threadIdx.x; q < AD * H; q += blockDim.x) base[q] = pa.w2[i][q];
+            for (int q = threadIdx.x; q < AD; q += blockDim.x) base[AD * H + q] = pa.b2[i][q];
         } else {
             for (int q = threadIdx.x; q < H * H; q += blockDim.x) base[q] = pa.w2[i][q];
             for (int q = threadIdx.x; q < H; q += blockDim.x) base[H * H + q] = pa.b2[i][q];
             base += H * H + H;
-            for (int q = threadIdx.x; q < 8 * H; q += blockDim.x)        // W3 [5][H] -> [H][8]
-                base[q] = (q & 7) < 5 ? pa.w3[i][(q & 7) * H + (q >> 3)] : 0.0f;
-            for (int q = threadIdx.x; q < 8; q += blockDim.x) base[8 * H + q] = q < 5 ? pa.b3[i][q] : 0.0f;
+            constexpr bool POW2 = (AP & (AP - 1)) == 0;   // every built program: AP = 4, 8 or 16
+            for (int q = threadIdx.x; q < AP * H; q += blockDim.x) {     // W3 [AD][H] -> [H][AP]
+                const int c = POW2 ? (q & (AP - 1)) : q % AP, r = POW2 ? (q >> ilog2(AP)) : q / AP;
+                base[q] = c < AD ? pa.w3[i][c * H + r] : 0.0f;
+            }
+            for (int q = threadIdx.x; q < AP; q += blockDim.x) base[AP * H + q] = q < AD ? pa.b3[i][q] : 0.0f;
         }
     });
     __syncthreads();
@@ -1021,6 +1084,10 @@ __global__ void __launch_bounds__(32 * kPolicyMaxWarps<DEPTH>) mpe_policy_rollou
         const float2 v = state_load(a.lm + l * n + wi);
         w.lx[l] = v.x; w.ly[l] = v.y;
     }
+    if constexpr (NC > 0) {   // the speakers' utterances of the previous step: what listeners observe at step 0
+#pragma unroll
+        for (int q = 0; q < NC; ++q) w.c[q] = a.comm[q * n + wi];
+    }
     if constexpr (P::G > 0) {
 #pragma unroll
         for (int q = 0; q < P::G; ++q) w.g[q] = a.goal[q * n + wi];
@@ -1048,16 +1115,21 @@ __global__ void __launch_bounds__(32 * kPolicyMaxWarps<DEPTH>) mpe_policy_rollou
             __syncwarp();   // every lane has streamed the tiles out before any lane refills them
         }
         float ux[A], uy[A];
+        float cact[NC > 0 ? NC : 1];
         static_for<A>([&](auto ic) {
-            constexpr int i = decltype(ic)::value;
+            constexpr int i = decltype(ic)::value, AD = P::act_dim(i);
             const float2 u = policy_agent<P, H, DEPTH, i>(d, w, s_w + PS::agent_off(i),
                                                           (pa.act_rec[i] != nullptr && active)
-                                                              ? pa.act_rec[i] + (static_cast<int64_t>(t) * n + wi) * 5 : nullptr,
-                                                          sample, pa.sample_key, gw, pa.sample_step + static_cast<uint32_t>(t));
+                                                              ? pa.act_rec[i] + (static_cast<int64_t>(t) * n + wi) * AD : nullptr,
+                                                          sample, pa.sample_key, gw, pa.sample_step + static_cast<uint32_t>(t),
+                                                          cact);
             ux[i] = u.x;
             uy[i] = u.y;
         });
         physics<P>(d, w, ux, uy);
+        // update_agent_state (core.py:172-178) after every agent has acted on the step-t utterances, as the fused step
+#pragma unroll
+        for (int q = 0; q < NC; ++q) w.c[q] = cact[q];
         float rew[A];
         P::reward(d, w, rew, nullptr);
         if (a.flags & MPE_FLAG_SHARED_REWARD) {
@@ -1078,6 +1150,8 @@ __global__ void __launch_bounds__(32 * kPolicyMaxWarps<DEPTH>) mpe_policy_rollou
 #pragma unroll
         for (int i = 0; i < A; ++i)
             if (P::movable(i)) a.pv[i * n + wi] = make_float4(w.px[i], w.py[i], w.vx[i], w.vy[i]);
+#pragma unroll
+        for (int q = 0; q < NC; ++q) a.comm[q * n + wi] = w.c[q];
     }
     if (active) {
 #pragma unroll
@@ -1094,11 +1168,18 @@ constexpr bool policy_rollout_ok() {     // every agent moves, nobody speaks: th
     for (int i = 0; i < P::A; ++i) ok = ok && P::movable(i) && P::act_dim(i) == 5;
     return ok;
 }
-// built for the BASELINE.json worlds (each instantiation unrolls obs_dim x H FMAs per agent: compile time)
-template <class P> struct PolicyBuilt { static constexpr bool value = false; };
-template <> struct PolicyBuilt<Simple<1, 1>> { static constexpr bool value = true; };
-template <> struct PolicyBuilt<Spread<3>> { static constexpr bool value = true; };
-template <> struct PolicyBuilt<Tag<3, 1, 2>> { static constexpr bool value = true; };
+// Worlds the closed loop is built for (each instantiation unrolls obs_dim x H FMAs per agent: compile time): the
+// BASELINE.json worlds (`baseline`: also the plain depth-1 kernel, and the opt-in step alternatives of make_program)
+// and the other scenarios of the MADDPG benchmark suite at their reference entity counts.
+template <class P> struct PolicyBuilt { static constexpr bool value = false, baseline = false; };
+template <> struct PolicyBuilt<Simple<1, 1>> { static constexpr bool value = true, baseline = true; };
+template <> struct PolicyBuilt<Spread<3>> { static constexpr bool value = true, baseline = true; };
+template <> struct PolicyBuilt<Tag<3, 1, 2>> { static constexpr bool value = true, baseline = true; };
+template <> struct PolicyBuilt<Adversary<1, 2, 2>> { static constexpr bool value = true, baseline = false; };
+template <> struct PolicyBuilt<Push<1, 1, 2>> { static constexpr bool value = true, baseline = false; };
+template <> struct PolicyBuilt<SpeakerListener> { static constexpr bool value = true, baseline = false; };
+template <> struct PolicyBuilt<Reference> { static constexpr bool value = true, baseline = false; };
+template <> struct PolicyBuilt<Crypto> { static constexpr bool value = true, baseline = false; };
 
 // ---- generic program for user scenarios (MPE_SCN_CUSTOM) ------------------------------------------
 // Any entity table, flags read at run time; same arithmetic primitives and the same (a, b) pair order as
@@ -1304,7 +1385,9 @@ struct Program {
     int pipe_smem;      // dynamic shared memory per WARP of the pipelined kernel
     void (*policy_fn[2][2])(PolicyArgs);  // K-step closed-loop rollout [depth - 1][hidden 32 / 64] (null: not built)
     void (*policy_plain_fn[2])(PolicyArgs);  // the same at depth 1 without exploration noise and observation records
+                                             // (null: policy_fn serves plain calls too)
     int policy_weight_floats[2][2];
+    bool policy_move_only;   // every agent moves and is silent: actions are the 5 movement probabilities (mpe_rollout_policy)
     void (*rollout_fn)(RolloutArgs);   // K-step open-loop rollout
     int rollout_smem;   // dynamic shared memory per WARP of the rollout kernel
     KernelFn lanes_fn;  // lane-per-agent fused step (simple_spread only), else null
@@ -1325,7 +1408,7 @@ static Program make_program() {
     p.fn[kObserve] = mpe_kernel<P, kObserve>;
     // the two restructurings that measurements rejected (warp pairs, software-pipelined persistent grid) stay available as
     // opt-in, bit-identical alternatives for the BASELINE.json worlds only (compile time)
-    constexpr bool kAlternatives = PolicyBuilt<P>::value || std::is_same<P, Spread<6>>::value ||
+    constexpr bool kAlternatives = PolicyBuilt<P>::baseline || std::is_same<P, Spread<6>>::value ||
                                    std::is_same<P, WorldComm<4, 2, 1, 2>>::value;
     if constexpr (kAlternatives && P::A >= 2 && pair_count<P>() * 64 <= Shape<P>::kWarpFloats - Shape<P>::obs_base())
         p.split_fn = mpe_kernel<P, kFusedStep, true>;     // (the pair exchange must fit the observation tiles)
@@ -1335,10 +1418,12 @@ static Program make_program() {
     p.pipe_smem = Shape<P>::kPipeWarpBytes;
     p.rollout_fn = mpe_rollout_kernel<P>;
     p.rollout_smem = Shape<P>::kRolloutWarpBytes;
-    // the closed-loop rollout is built for the BASELINE.json scenarios whose agents all move and are silent
-    if constexpr (policy_rollout_ok<P>() && PolicyBuilt<P>::value) {
-        p.policy_plain_fn[0] = mpe_policy_rollout_kernel<P, 32, 1, false>;
-        p.policy_plain_fn[1] = mpe_policy_rollout_kernel<P, 64, 1, false>;
+    // the closed-loop rollout; only the BASELINE.json worlds also get the plain depth-1 build (compile time)
+    if constexpr (PolicyBuilt<P>::value) {
+        if constexpr (PolicyBuilt<P>::baseline) {
+            p.policy_plain_fn[0] = mpe_policy_rollout_kernel<P, 32, 1, false>;
+            p.policy_plain_fn[1] = mpe_policy_rollout_kernel<P, 64, 1, false>;
+        }
         p.policy_fn[0][0] = mpe_policy_rollout_kernel<P, 32, 1, true>;
         p.policy_fn[0][1] = mpe_policy_rollout_kernel<P, 64, 1, true>;
         p.policy_fn[1][0] = mpe_policy_rollout_kernel<P, 32, 2, true>;
@@ -1348,6 +1433,7 @@ static Program make_program() {
         p.policy_weight_floats[1][0] = PolicyShape<P, 32, 2>::kWeightFloats;
         p.policy_weight_floats[1][1] = PolicyShape<P, 64, 2>::kWeightFloats;
     }
+    p.policy_move_only = policy_rollout_ok<P>();
     p.smem_bytes = Shape<P>::kWarpBytes;  // per warp
     p.A = P::A; p.L = P::L; p.NS = P::NS; p.DIMC = P::DIMC; p.INFO = P::INFO; p.G = P::G;
     for (int i = 0; i < P::A; ++i) { p.obs_dim[i] = P::obs_dim(i); p.act_dim[i] = P::act_dim(i); }
@@ -1928,6 +2014,12 @@ static int policy_warps_per_block(mpe_handle h, int di, int k, int64_t warps) {
     return wpb;
 }
 
+extern "C" int mpe_collect_supported(mpe_handle h, int32_t depth, int32_t hidden) {
+    if (!h || (depth != 1 && depth != 2) || (hidden != 32 && hidden != 64)) return MPE_ERR_BAD_ARG;
+    const bool built = h->prog->scenario != MPE_SCN_CUSTOM && h->prog->policy_fn[depth - 1][hidden == 32 ? 0 : 1] != nullptr;
+    return built ? MPE_OK : MPE_ERR_UNSUPPORTED;
+}
+
 extern "C" int mpe_collect(mpe_handle h, void *pv, const void *lm, float *comm, const int32_t *goal, int32_t depth,
                            int32_t hidden, const float *const *w1_n, const float *const *b1_n, const float *const *w2_n,
                            const float *const *b2_n, const float *const *w3_n, const float *const *b3_n, int32_t n_steps,
@@ -1946,9 +2038,10 @@ extern "C" int mpe_collect(mpe_handle h, void *pv, const void *lm, float *comm, 
         if (act_record_n && act_record_n[i] != nullptr && !ok4(act_record_n[i])) return MPE_ERR_BAD_ARG;
         if (obs_record_n && !ok16(obs_record_n[i])) return MPE_ERR_BAD_ARG;
     }
+    if (h->prog->NS * h->prog->DIMC > 0 && !ok4(comm)) return MPE_ERR_BAD_ARG;
     if (h->device < 0) return MPE_ERR_NO_DEVICE;
     const int di = depth - 1, k = hidden == 32 ? 0 : 1;
-    if (h->prog->scenario == MPE_SCN_CUSTOM || h->prog->policy_fn[di][k] == nullptr) return MPE_ERR_UNSUPPORTED;
+    if (mpe_collect_supported(h, depth, hidden) != MPE_OK) return MPE_ERR_UNSUPPORTED;
     if (flags & (MPE_FLAG_DISCRETE_ACTION_INPUT | MPE_FLAG_FORCE_DISCRETE_ACTION)) return MPE_ERR_UNSUPPORTED;
     NvtxRange range("mpe_collect");
     PolicyArgs pa{};
@@ -1984,7 +2077,8 @@ extern "C" int mpe_collect(mpe_handle h, void *pv, const void *lm, float *comm, 
     cudaError_t e = cudaErrorInvalidValue;
     if (blocks <= 0x7fffffffLL) {
         void *params[] = {&pa};
-        const bool plain = depth == 1 && !(flags & MPE_FLAG_SAMPLE_ACTIONS) && obs_record_n == nullptr;
+        const bool plain = depth == 1 && !(flags & MPE_FLAG_SAMPLE_ACTIONS) && obs_record_n == nullptr &&
+                           h->prog->policy_plain_fn[k] != nullptr;
         e = cudaLaunchKernel(reinterpret_cast<const void *>(plain ? h->prog->policy_plain_fn[k] : h->prog->policy_fn[di][k]),
                              dim3(static_cast<unsigned>(blocks)),
                              dim3(32 * wpb), params, static_cast<size_t>(policy_smem_bytes(h->prog, di, k, wpb)),
@@ -2005,7 +2099,7 @@ extern "C" int mpe_rollout_policy(mpe_handle h, void *pv, const void *lm, float 
     if (!h || n_steps < 0 || !w1_n || !b1_n || !w2_n || !b2_n) return MPE_ERR_BAD_ARG;
     if (h->device < 0) return MPE_ERR_NO_DEVICE;
     const int k = hidden == 32 ? 0 : (hidden == 64 ? 1 : -1);
-    if (k < 0 || h->prog->scenario == MPE_SCN_CUSTOM || h->prog->policy_fn[0][k] == nullptr) return MPE_ERR_UNSUPPORTED;
+    if (k < 0 || mpe_collect_supported(h, 1, hidden) != MPE_OK || !h->prog->policy_move_only) return MPE_ERR_UNSUPPORTED;
     return mpe_collect(h, pv, lm, comm, goal, 1, hidden, w1_n, b1_n, w2_n, b2_n, nullptr, nullptr, n_steps, 0, 0, 0,
                        obs_n, rew_sum, rew_steps, act_record_n, nullptr, done, flags & ~MPE_FLAG_SAMPLE_ACTIONS, stream);
 }

@@ -243,23 +243,27 @@ class MultiAgentEnv(_Env):
     def rollout_policy(self, policies, n_steps, record_actions=False, per_step_rewards=False, record_observations=False,
                        explore_seed=None, explore_step=0):
         """T closed-loop steps in ONE kernel launch with the actors inside the kernel (mpe_collect).  policies[i] is agent
-        i's actor, H = 32 or 64, the same depth and H for every agent:
-          one hidden layer   a_i = softmax(W2_i relu(W1_i obs_i + b1_i) + b2_i): a `torch.nn.Sequential(Linear(obs_dim_i,
-              H), ReLU(), Linear(H, 5))` or the tuple (W1 [H, obs_dim_i], b1 [H], W2 [5, H], b2 [5]);
-          two hidden layers (the MADDPG actor) a_i = softmax(W3_i relu(W2_i relu(W1_i obs_i + b1_i) + b2_i) + b3_i): a
-              `torch.nn.Sequential(Linear(obs_dim_i, H), ReLU(), Linear(H, H), ReLU(), Linear(H, 5))` or the tuple
-              (W1, b1, W2 [H, H], b2 [H], W3 [5, H], b3 [5]);
-        all in torch's Linear layout.  explore_seed=None acts with softmax(logits); an int acts with MADDPG's exploration
-        sample softmax(logits - log(-log u)), u uniform in (0, 1) drawn from a Philox stream keyed by (explore_seed,
-        global world index, explore_step + t, agent): a sharded env draws what the full batch draws, and a rollout split
-        into calls with explore_step = 0, T1, T1 + T2, ... draws what one call does.
+        i's actor with A_i = act_dim_i = action_space[i]'s width outputs, H = 32 or 64, the same depth and H for every
+        agent:
+          one hidden layer   logits_i = W2_i relu(W1_i obs_i + b1_i) + b2_i: a `torch.nn.Sequential(Linear(obs_dim_i,
+              H), ReLU(), Linear(H, A_i))` or the tuple (W1 [H, obs_dim_i], b1 [H], W2 [A_i, H], b2 [A_i]);
+          two hidden layers (the MADDPG actor) logits_i = W3_i relu(W2_i relu(W1_i obs_i + b1_i) + b2_i) + b3_i: a
+              `torch.nn.Sequential(Linear(obs_dim_i, H), ReLU(), Linear(H, H), ReLU(), Linear(H, A_i))` or the tuple
+              (W1, b1, W2 [H, H], b2 [H], W3 [A_i, H], b3 [A_i]);
+        all in torch's Linear layout.  The logits are the heads of the agent's action space, as MADDPG splits them: 5
+        movement logits if the agent moves, then dim_c communication logits if it speaks; each head gets its own
+        softmax, and the comm head's probabilities are what the agent says.  explore_seed=None acts with
+        softmax(logits); an int acts with MADDPG's exploration sample softmax(logits - log(-log u)) per head, u uniform in
+        (0, 1) drawn from a Philox stream keyed by (explore_seed, global world index, explore_step + t, agent, logit): a
+        sharded env draws what the full batch draws, and a rollout split into calls with explore_step = 0, T1, T1 + T2,
+        ... draws what one call does.
         Returns (obs_n, reward_sum_n, done_n, info_n, extras) for the state after the last step; extras["actions"]
-        (record_actions) is a list of [T, N, 5] tensors with the actions taken, extras["rewards"] (per_step_rewards) a
+        (record_actions) is a list of [T, N, A_i] tensors with the actions taken, extras["rewards"] (per_step_rewards) a
         [T, n, N] tensor, extras["observations"] (record_observations) a list of [T, N, obs_dim_i] tensors whose row t is
         the observation agent i acted on at step t -- with the final obs_n, the (obs, act, rew, next obs) of every step.
-        World state lives in registers for all T steps.  Batched CUDA mode; scenarios whose agents all move and are
-        silent and whose program was built with the policy kernel (simple, simple_spread N=3, simple_tag 3+1) --
-        anything else raises."""
+        World state lives in registers for all T steps.  Batched CUDA mode; scenarios whose program was built with the
+        policy kernel (simple, simple_spread N=3, simple_tag 3+1, simple_adversary 1+2, simple_push,
+        simple_speaker_listener, simple_reference, simple_crypto) -- anything else raises MpeError."""
         import torch
         world = self.world
         if not world.batched:
@@ -278,7 +282,10 @@ class MultiAgentEnv(_Env):
             if explore_step < 0 or explore_step + T >= 2 ** 32:
                 raise ValueError("explore_step + n_steps must stay below 2**32 (the step counter of the noise stream)")
             flags |= _lib.FLAG_SAMPLE_ACTIONS
-        depth, hidden, params = actor_parameters(policies, nw.obs_dims)
+        # a scenario without the kernel is refused before the actors are looked at: their shapes mean nothing there
+        if all(nw.collect_supported(d, h) != 0 for d in (1, 2) for h in (32, 64)):
+            _lib.check(_lib.ERR_UNSUPPORTED, "rollout_policy (mpe_collect_supported)")
+        depth, hidden, params = actor_parameters(policies, nw.obs_dims, nw.act_dims)
         keep = []
         for W in params:
             W = [t.detach().to(device=nw.device, dtype=torch.float32) for t in W]
@@ -287,7 +294,8 @@ class MultiAgentEnv(_Env):
         ptrs = [_lib.ptr_array([W[k].data_ptr() for W in keep]) if k < len(keep[0]) else None for k in range(6)]
         out = nw.out if self.reuse_buffers else nw.new_outputs()
         rew_steps = torch.empty((T, self.n, N), dtype=torch.float32, device=nw.device) if per_step_rewards else None
-        actions = [torch.empty((T, N, 5), dtype=torch.float32, device=nw.device) for _ in range(self.n)] if record_actions else None
+        actions = [torch.empty((T, N, ad), dtype=torch.float32, device=nw.device)
+                   for ad in nw.act_dims] if record_actions else None
         observations = [torch.empty((T, N, od), dtype=torch.float32, device=nw.device)
                         for od in nw.obs_dims] if record_observations else None
         nw.collect(depth, hidden, ptrs, T, out, flags, explore_seed or 0, explore_step if explore_seed is not None else 0,
@@ -556,12 +564,15 @@ class MultiAgentEnv(_Env):
         return results
 
 
-def actor_parameters(policies, obs_dims):
+def actor_parameters(policies, obs_dims, act_dims=None):
     """(depth, H, [per-agent weight tuples in torch's Linear layout]) of the actors MultiAgentEnv.rollout_policy runs:
     depth 1 -- a module holding exactly two Linear layers (Linear -> ReLU -> Linear) or (W1, b1, W2, b2); depth 2 -- a
     `Sequential(Linear, ReLU, Linear, ReLU, Linear)` or (W1, b1, W2, b2, W3, b3).  Every agent must have the same depth
-    and H, and the shapes must fit its observation; anything else raises ValueError.  Works on tensors of any device."""
+    and H, and the shapes must fit its observation and its action width act_dims[i] (None: 5 for every agent, the
+    movement head alone); anything else raises ValueError.  Works on tensors of any device."""
     import torch
+    if act_dims is None:
+        act_dims = [5] * len(policies)
     depth = hidden = None
     params = []
     for i, pol in enumerate(policies):
@@ -584,8 +595,9 @@ def actor_parameters(policies, obs_dims):
             depth, hidden = d, H
         if d != depth:
             raise ValueError("policy %d has %d hidden layers, policy 0 has %d: all actors must have the same depth" % (i, d, depth))
-        want = [(hidden, obs_dims[i]), (hidden,)] + ([(5, hidden), (5,)] if depth == 1 else
-                                                      [(hidden, hidden), (hidden,), (5, hidden), (5,)])
+        ad = int(act_dims[i])
+        want = [(hidden, obs_dims[i]), (hidden,)] + ([(ad, hidden), (ad,)] if depth == 1 else
+                                                      [(hidden, hidden), (hidden,), (ad, hidden), (ad,)])
         if [tuple(t.shape) for t in pol] != want:
             raise ValueError("policy %d: expected shapes %s, got %s" % (i, want, [tuple(t.shape) for t in pol]))
         params.append(pol)

@@ -41,6 +41,11 @@ class ShapeHandle(object):
         self.bytes_per_env_step = lib.mpe_bytes_per_env_step(h)
         self._speakers = [i for i in range(self.n_agents) if not desc.agent_silent[i]]
 
+    def collect_supported(self, depth, hidden):
+        """mpe_collect_supported: 0 if mpe_collect is built for this scenario at (depth, hidden), else
+        _lib.ERR_UNSUPPORTED (ERR_BAD_ARG for a depth or width the kernel never takes)"""
+        return self.lib.mpe_collect_supported(self.handle, int(depth), int(hidden))
+
     def speaker_slot(self, agent_index):
         """row block of agent `agent_index` in the comm tensors, or -1 if the agent is silent"""
         try:

@@ -27,15 +27,29 @@ def card():
     return {"name": torch.cuda.get_device_name(0), "power_limit": limit}
 
 
-def actors(obs_dims, H, depth, dev):
+def actors(obs_dims, act_dims, H, depth, dev):
     import torch
     nn = torch.nn
     torch.manual_seed(0)
     mods = []
-    for od in obs_dims:
-        layers = [nn.Linear(od, H), nn.ReLU()] + ([nn.Linear(H, H), nn.ReLU()] if depth == 2 else []) + [nn.Linear(H, 5)]
+    for od, ad in zip(obs_dims, act_dims):
+        layers = [nn.Linear(od, H), nn.ReLU()] + ([nn.Linear(H, H), nn.ReLU()] if depth == 2 else []) + [nn.Linear(H, ad)]
         mods.append(nn.Sequential(*layers).to(dev))
     return mods
+
+
+def action_heads(nw):
+    """per agent, the column ranges of its action heads: 5 movement logits if it moves, then dim_c if it speaks"""
+    heads = []
+    for i in range(nw.n_agents):
+        h, c = [], 0
+        if nw.desc.agent_movable[i]:
+            h.append((0, 5))
+            c = 5
+        if not nw.desc.agent_silent[i]:
+            h.append((c, c + nw.dim_c))
+        heads.append(h)
+    return heads
 
 
 def time_calls(fn, reps, stream=None):
@@ -62,7 +76,8 @@ def measure(scenario, n, T, depth, H, sample, record, reps, dev):
     env.reuse_buffers = True
     env.reset()
     nw = env.world.native
-    mods = actors(nw.obs_dims, H, depth, dev)
+    mods = actors(nw.obs_dims, nw.act_dims, H, depth, dev)
+    heads = action_heads(nw)
     kw = dict(record_actions=record, per_step_rewards=record, record_observations=record)
     if sample:
         kw["explore_seed"] = 1
@@ -73,7 +88,7 @@ def measure(scenario, n, T, depth, H, sample, record, reps, dev):
     A = len(mods)
     rec = None
     if record:
-        rec = dict(act=[torch.empty(T, n, 5, device=dev) for _ in range(A)],
+        rec = dict(act=[torch.empty(T, n, ad, device=dev) for ad in nw.act_dims],
                    obs=[torch.empty(T, n, od, device=dev) for od in nw.obs_dims],
                    rew=torch.empty(T, A, n, device=dev))
     clock = {"t": 0}
@@ -87,7 +102,10 @@ def measure(scenario, n, T, depth, H, sample, record, reps, dev):
             if sample:
                 u = torch.rand_like(logits)
                 logits = logits - torch.log(-torch.log(u))
-            a = torch.softmax(logits, -1)
+            if len(heads[i]) == 1:
+                a = torch.softmax(logits, -1)
+            else:     # one Gumbel-softmax per head, as MADDPG samples a MultiDiscrete action
+                a = torch.cat([torch.softmax(logits[:, lo:hi], -1) for lo, hi in heads[i]], -1)
             if rec is not None:
                 rec["obs"][i][t].copy_(o)
                 rec["act"][i][t].copy_(a)
@@ -113,7 +131,9 @@ def measure(scenario, n, T, depth, H, sample, record, reps, dev):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--scenarios", default="simple_spread,simple_tag")
+    ap.add_argument("--scenarios", default="simple_spread,simple_tag",
+                    help="comma-separated, any of simple, simple_spread, simple_tag, simple_adversary, simple_push, "
+                         "simple_speaker_listener, simple_reference, simple_crypto")
     ap.add_argument("--num-envs", type=int, default=65536)
     ap.add_argument("--steps", type=int, default=25)
     ap.add_argument("--hidden", type=int, default=64)
